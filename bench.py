@@ -2,6 +2,7 @@
 """Benchmark of the per-frame rendering hot path (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload C2|C1|C4]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one boosted frame (`Network.forward`) of the configuration BASELINE.json's metric is
@@ -50,7 +51,40 @@ def parse_args():
                     help="skip timing the reference's op sequence (oracle restatement) as eager PyTorch on this GPU (N=1 leg)")
     ap.add_argument("--no-strict", action="store_true", help="skip the strict-fp32 timing / parity legs")
     ap.add_argument("--ref-budget-s", type=float, default=300.0, help="time budget of the --impl reference run")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (a fixed sample above 64 MB in all)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        # the reference arm picks its frame size from a time budget: its outputs are not the same from run to run
+        ap.error("--dump-outputs writes the outputs of --impl ours")
+    return args
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(dump_dir, outs, limit=DUMP_LIMIT_BYTES):
+    """Writes every tensor of `outs` (the outputs of the last timed step) as dump_dir/<name>.npy, float32 (float64 for
+    integer or boolean outputs), so that two builds run with the same arguments can be compared output for output.
+    Above `limit` bytes in all, every array is cut to a fixed, seeded sample of its flattened elements (the same sample
+    for the same shapes) holding the same fraction of each array."""
+    import numpy as np
+    import torch
+    arrays = {}
+    for k, v in outs.items():
+        if not torch.is_tensor(v):
+            continue
+        v = v.detach().cpu()
+        arrays[k] = v.float().numpy() if v.is_floating_point() else v.double().numpy()
+    total = sum(a.nbytes for a in arrays.values())
+    os.makedirs(dump_dir, exist_ok=True)
+    for k, a in sorted(arrays.items()):
+        if total > limit:
+            m = max(1, a.size * limit // total)
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, m, replace=False))]
+        np.save(os.path.join(dump_dir, f"{k}.npy"), a)
 
 
 # ------------------------------------------------------------------------------------------ clocks
@@ -430,6 +464,7 @@ def main_ours(args):
     t_host = (time.time() - t_wall0) / args.steps * 1e3        # host time to ENQUEUE one frame
     barrier()
     t_wall1 = time.time()
+    eager_out = {k: v.detach().cpu() for k, v in out.items()} if args.dump_outputs else None
     launches = (_lib.launch_count() - l0) / args.steps
     ms = max_over_ranks(e0.elapsed_time(e1) / args.steps)
     clk = clocks.stop(t_wall0, t_wall1)
@@ -721,9 +756,11 @@ def main_ours(args):
              "e2e_value": world * rays_per_frame / (ms_e2e * 1e-3)}
     # headline = the faster of the two public entry points (Network.forward / FrameGraph.__call__), chosen
     # separately for the device-resident number and for the end-to-end number; both modes are listed in full
-    execution = "value: eager (stream launches)"
+    execution, timed_out = "value: eager (stream launches)", eager_out
     if graph_res and "error" not in graph_res and graph_res["ms_per_step"] < ms:
-        ms, execution = graph_res["ms_per_step"], "value: cuda_graph replay (FrameGraph)"
+        ms, execution, timed_out = graph_res["ms_per_step"], "value: cuda_graph replay (FrameGraph)", default_out
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, timed_out)
     if graph_res and "error" not in graph_res and graph_res["e2e_ms_per_step"] < ms_e2e:
         ms_e2e, execution = graph_res["e2e_ms_per_step"], execution + "; e2e: cuda_graph replay (FrameGraph)"
     else:
@@ -941,6 +978,8 @@ def main_mvs(args):
     e1.record()
     barrier()
     tw1 = time.time()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out)
     ms = e0.elapsed_time(e1) / args.steps
     launches = (_lib.launch_count() - l0) / args.steps
     clk = clocks.stop(tw0, tw1)

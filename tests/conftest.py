@@ -10,6 +10,9 @@ if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
 GOLDEN_DIR = os.path.join(ROOT, "tests", "golden")
+# Intra-op threads of the process that wrote the golden vectors (oracle/gen_golden.py).  MKL splits a GEMM by thread
+# count, so the CPU oracle reproduces the reference's outputs bit for bit only with the same count.
+GOLDEN_INTRA_OP_THREADS = 8
 
 
 def pytest_configure(config):
@@ -65,3 +68,12 @@ def load_golden(name):
 @pytest.fixture(scope="session")
 def ops_golden():
     return load_golden("enerf_ops.npz")
+
+
+@pytest.fixture
+def golden_threads():
+    """Runs a test with the intra-op thread count the golden vectors were written with."""
+    old = torch.get_num_threads()
+    torch.set_num_threads(GOLDEN_INTRA_OP_THREADS)
+    yield
+    torch.set_num_threads(old)

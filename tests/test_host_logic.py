@@ -3,7 +3,6 @@ inference plan, refusal paths, benchmark byte model.  No kernel is launched here
 import ctypes
 import os
 import re
-import subprocess
 import sys
 
 import numpy as np
@@ -187,28 +186,68 @@ def test_bench_byte_model_matches_survey():
     assert alg["composite_blend_l1"] == 112803840       # 113 MB (216 B/ray)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/lib"), reason="reference tree not present")
-def test_plugin_loads_through_the_reference_factory():
-    code = r'''
-import os, sys
-sys.path.insert(0, %r)
-from oracle.ref_loader import load_reference
-ns = load_reference(opts=["enerf.cas_config.k_best", 2, "network_module", "boostmvsnerfs_b200.reference_plugin.boost_enerf"])
-os.chdir(%r)
-from lib.networks.make_network import make_network
-net = make_network(ns["cfg"], preprocess=True)
-ref = ns["boost_enerf_network"].Network(preprocess=True)
-net.load_state_dict(ref.state_dict(), strict=True)
-assert net.rc.k_best == 2 and net.rc.render_if == (False, True)
-try:
-    make_network(ns["cfg"])
-    raise SystemExit("expected FileNotFoundError")
-except FileNotFoundError:
-    pass
-print("PLUGIN_OK")
-''' % (ROOT, ROOT)
-    out = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=300)
-    assert "PLUGIN_OK" in out.stdout, out.stdout[-2000:] + out.stderr[-2000:]
+def test_bench_dump_outputs_writes_float_arrays_and_a_fixed_sample_above_the_limit(tmp_path):
+    import bench
+    g = torch.Generator().manual_seed(0)
+    outs = {"rgb": torch.rand(1, 1000, 3, generator=g).half(), "depth": torch.rand(1, 1000, generator=g),
+            "count": torch.arange(7), "_size": (4, 5)}
+    bench.dump_outputs(str(tmp_path / "whole"), outs)
+    for k in ("rgb", "depth", "count"):
+        a = np.load(tmp_path / "whole" / f"{k}.npy")
+        assert a.dtype == (np.float64 if k == "count" else np.float32)
+        assert np.array_equal(a, outs[k].double().numpy())
+    assert sorted(os.listdir(tmp_path / "whole")) == ["count.npy", "depth.npy", "rgb.npy"]
+    limit = 4000                                        # below the 16056 B of the three arrays as dumped
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), outs, limit=limit)
+    total = 0
+    for k in ("rgb", "depth", "count"):
+        a, b = np.load(tmp_path / "a" / f"{k}.npy"), np.load(tmp_path / "b" / f"{k}.npy")
+        assert np.array_equal(a, b) and a.ndim == 1 and 0 < a.size < outs[k].numel()
+        assert np.isin(a, outs[k].double().numpy().reshape(-1)).all()
+        total += a.nbytes
+    assert total <= limit
+
+
+class _YacsNode(dict):
+    """Attribute access over a dict, like the reference's yacs CfgNode."""
+    __getattr__ = dict.__getitem__
+
+
+def test_plugin_loads_through_the_reference_factory(tmp_path, monkeypatch):
+    """The plugin file loaded the way the reference's factory loads a network: imp.load_source(cfg.network_module,
+    cfg.network_path).Network([preprocess]) (reference lib/networks/make_network.py:3-10), network_path being the module
+    name as a path relative to the CWD (reference lib/config/config.py:166-168).  The reference's global config module
+    `lib.config` is stood in for by the evaluate/enerf_ours values with enerf.cas_config.k_best 2; the network must load
+    the reference network's own state dict under that config (the sd_* arrays of tests/golden/enerf_chain_eval.npz)
+    strictly, and without pre-processing it needs <result_dir>/view_selection.json like the reference."""
+    import dataclasses
+    import json
+    import types
+    monkeypatch.syspath_prepend(os.path.join(ROOT, "oracle", "shims"))
+    import imp                                                   # the shim of the stdlib module the factory uses
+    from conftest import load_golden
+    rc = dataclasses.asdict(RenderConfig.enerf_eval(2))
+    top = ("cost_volume_input_views", "chunk_size", "white_bkgd", "viewdir_agg")
+    module = "boostmvsnerfs_b200.reference_plugin.boost_enerf"
+    cfg = _YacsNode(network_module=module, network_path=module.replace(".", "/") + ".py", result_dir=str(tmp_path),
+                    enerf=_YacsNode({k: rc[k] for k in top}, cas_config=_YacsNode({k: v for k, v in rc.items() if k not in top})))
+    monkeypatch.setitem(sys.modules, "lib", types.ModuleType("lib"))
+    monkeypatch.setitem(sys.modules, "lib.config", types.SimpleNamespace(cfg=cfg))
+    monkeypatch.delitem(sys.modules, module, raising=False)
+    monkeypatch.chdir(ROOT)
+
+    def make_network(cfg, *args):
+        return imp.load_source(cfg.network_module, cfg.network_path).Network(*args)
+
+    net = make_network(cfg, True)
+    g = load_golden("enerf_chain_eval.npz")
+    net.load_state_dict({k[3:]: g.t(k) for k in g.keys() if k.startswith("sd_")}, strict=True)
+    assert net.rc.k_best == 2 and net.rc.render_if == (False, True)
+    with pytest.raises(FileNotFoundError):
+        make_network(cfg)
+    (tmp_path / "view_selection.json").write_text(json.dumps({"synth_0": [1, 2]}))
+    assert make_network(cfg).view_selection_outputs == {"synth_0": [1, 2]}
 
 
 def test_sinks_oracle_arithmetic():

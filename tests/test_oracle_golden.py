@@ -10,6 +10,7 @@ from boostmvsnerfs_b200.modules import EnerfModules
 from conftest import load_golden
 from oracle import enerf_oracle as O
 
+pytestmark = pytest.mark.usefixtures("golden_threads")
 RC = RenderConfig.enerf_eval(k_best=2)
 H, W = 64, 96
 

@@ -8,6 +8,7 @@ from boostmvsnerfs_b200.modules_mvs import MvsnerfModules, MvsNerfMlp
 from conftest import load_golden
 from oracle import mvsnerf_oracle as M
 
+pytestmark = pytest.mark.usefixtures("golden_threads")
 H, W = 64, 96
 
 
