@@ -23,9 +23,9 @@ def test_chain_blocks_and_slabs():
             assert sorted(k for a, b in blocks for k in range(a, b)) == list(range(K))
             assert all(blocks[i][1] == blocks[i + 1][0] or blocks[i + 1] == (K, K) for i in range(g - 1))
     # every row a ray reads through the fp32 align_corners mapping lies inside its rank's slab
-    for H, hv in ((544, 272), (1088, 544), (96, 48), (64, 8), (33, 17)):
+    for H, hv in ((544, 272), (1088, 544), (96, 48), (64, 8), (33, 17), (66, 33)):
         scale = np.float32(hv - 1) / np.float32(H - 1)
-        for g in (1, 2, 3, 8):
+        for g in (1, 2, 3, 4, 8):
             for r in range(g):
                 t0, t1 = bdist.row_tile(H, g, r)
                 y0, y1 = bdist.slab_rows(t0, t1, H, hv)
@@ -35,6 +35,14 @@ def test_chain_blocks_and_slabs():
                 i1 = np.minimum(i0 + 1, hv - 1)
                 if len(rows):
                     assert i0.min() >= y0 and i1.max() < y1, (H, hv, g, r)
+                # the trilinear volume fetch (lean_gather.cuh) reaches its rows through grid_sample's normalisation
+                # instead, each op rounded to fp32: iy = ((y / (H-1) * 2 - 1 + 1) * 0.5) * (hv-1), rows floor(iy) and +1
+                gy = rows / np.float32(H - 1) * np.float32(2) - np.float32(1)
+                iy = (gy + np.float32(1)) * np.float32(0.5) * np.float32(hv - 1)
+                f0 = np.floor(iy).astype(np.int64)
+                f1 = np.minimum(f0 + 1, hv - 1)
+                if len(rows):
+                    assert f0.min() >= y0 and f1.max() < y1, (H, hv, g, r)
             assert sum(b - a for a, b in (bdist.slab_rows(*bdist.row_tile(H, g, q), H, hv) for q in range(g))) <= hv + 4 * g
 
 

@@ -4,6 +4,8 @@ Two bars:  (1) with operands that are exactly representable in fp16 the kernel's
 fp32 convolution is summation order -> 1e-5 relative;  (2) with arbitrary fp32 operands the fp16 operand
 rounding gives TF32-class error -> 2e-3 of the output scale (tolerances per north_star: 1e-2 wherever
 reduced-precision operands are enabled)."""
+import math
+
 import pytest
 import torch
 
@@ -309,6 +311,93 @@ def test_conv3d_k3_umma_matches_cudnn(shape, exact_operands):
     assert (got.float() - ref).abs().max().item() <= tol, ((got.float() - ref).abs().max().item(), scale)
     old = ops.conv3d_k3(xh, pack_conv3d_k3(w), b, Cout, relu)
     assert (got.float() - old).abs().max().item() <= max(tol, 2e-5 * scale)
+
+
+UMMA_TILE = {8: (4, 4, 126), 16: (2, 4, 128)}           # (TD, TH, TW) of bmv_conv3d_k3_umma per Cin (conv3d_umma.cu)
+UMMA_SMS = 148                                          # persistent grid: min(tiles, 148) CTAs
+UMMA_MODE_COUT = {0: 9, 1: 8, 2: 16, 3: 12}
+
+
+def _umma_tiles(cin, dhw):
+    return math.prod(-(-n // t) for n, t in zip(dhw, UMMA_TILE[cin]))
+
+
+def _umma_in_mode(x, wfrag, b, mode):
+    """bmv_conv3d_k3_umma with an output layout that selects epilogue `mode` (conv3d_umma.cu): 0 fp32 features + channel
+    8 to out2 (the merged heads), 1 fp16 with 8 channels, 2 fp32 with 16 channels, 3 per-element stores (here 12
+    channels into a channel slice of a wider tensor).  Returns every output channel, and for mode 3 the whole wider
+    tensor, so that stray writes into the channels around the slice are compared too."""
+    from boostmvsnerfs_b200 import ops
+    N, _, D, H, W = x.shape
+    cout = UMMA_MODE_COUT[mode]
+    if mode == 0:
+        out2 = torch.empty((N, 1, D, H, W), device="cuda")
+        return torch.cat([ops.conv3d_k3(x, wfrag, b, cout, False, out2=out2, split=8, engine="umma"), out2], dim=1)
+    if mode == 1:
+        return ops.conv3d_k3(x, wfrag, b, cout, True, out_dtype=torch.float16, engine="umma")
+    if mode == 2:
+        return ops.conv3d_k3(x, wfrag, b, cout, False, engine="umma")
+    big = torch.full((N, 16, D, H, W), -7.0, device="cuda").contiguous(memory_format=torch.channels_last_3d)
+    ops.conv3d_k3(x, wfrag, b, cout, True, out=big[:, 2:14], engine="umma")
+    return big
+
+
+@pytest.mark.parametrize("cin,dhw,batches", [
+    (8, (4, 4, 126), (147, 148, 149, 296, 297, 445, 600)),      # one tile per volume
+    (8, (3, 3, 100), (147, 148, 149, 296, 297, 445, 600)),      # one tile, ragged in every dimension
+    (16, (2, 4, 128), (147, 148, 149, 296, 297, 445, 600)),
+    (16, (1, 3, 77), (147, 148, 149, 296, 297, 445, 600)),
+    (8, (8, 32, 252), (16,)),                                   # 32 tiles per volume: 512 tiles
+], ids=["cin8", "cin8-ragged", "cin16", "cin16-ragged", "cin8-32-tiles-per-volume"])
+@pytest.mark.parametrize("mode", [0, 1, 2, 3])
+def test_conv3d_k3_umma_is_batch_independent(cin, dhw, batches, mode):
+    """bmv_conv3d_k3_umma is persistent: min(tiles, 148) CTAs walk tiles blockIdx.x, +148, ... through a 2-slot ring (a
+    staged TMA tile + a TMEM accumulator set per slot; slot = it % 2, mbarrier parity (it / 2) & 1).  A tile's MMAs and
+    epilogue do not depend on the slot or the CTA that runs them, so a launch over N volumes must equal, bit for bit,
+    launches over chunks of at most 148 tiles, in which every CTA runs exactly one tile.  With one-tile volumes, tile t
+    is volume t and N covers one partial wave (147), the full wave (148), slot 1 first used (149), slot 0 reused with
+    its parity flipped (297), several flips (445, 600) and ragged last waves.  Every epilogue mode is covered."""
+    from boostmvsnerfs_b200.mlp_pack import pack_conv3d_k3_umma
+    per_vol = _umma_tiles(cin, dhw)
+    assert max(batches) * per_vol > 2 * UMMA_SMS               # some CTA runs >= 3 tiles (slot 0 twice)
+    chunk = max(1, UMMA_SMS // per_vol)                        # volumes per reference launch: <= 148 tiles
+    cout = UMMA_MODE_COUT[mode]
+    g = torch.Generator().manual_seed(cin * 1000 + dhw[2] * 10 + mode)
+    x = torch.randn((max(batches), cin, *dhw), generator=g).half().cuda().contiguous(memory_format=torch.channels_last_3d)
+    w = (torch.randn((cout, cin, 3, 3, 3), generator=g) * 0.1).cuda()
+    b = torch.randn(cout, generator=g).cuda()
+    wfrag = pack_conv3d_k3_umma(w)
+    for N in batches:
+        xs = x[:N]
+        full = _umma_in_mode(xs, wfrag, b, mode)
+        ref = torch.cat([_umma_in_mode(xs[i:i + chunk], wfrag, b, mode) for i in range(0, N, chunk)])
+        assert full.abs().max().item() > 0
+        if mode == 3:
+            assert bool((full[:, :2] == -7.0).all()) and bool((full[:, 14:] == -7.0).all()), f"N={N}: write outside the slice"
+        diff = (full.float() - ref.float()).abs()
+        assert torch.equal(full, ref), (f"N={N} ({N * per_vol} tiles): {int((diff > 0).sum())} outputs differ from the "
+                                        f"one-tile-per-CTA launches, max {diff.max().item():.3e}")
+
+
+@pytest.mark.parametrize("shape", [(4, 8, 9, 64, 68, 120), (4, 8, 9, 8, 272, 480)], ids=["level0", "level1"])
+def test_conv3d_k3_umma_merged_heads_at_frame_size(shape):
+    """The merged U-Net heads of a C2 frame (K = 4 chains, 960x544): level 0 is 1088 tiles, level 1 2176 (7 to 15 per
+    CTA).  fp16-representable operands, so the only difference from a float64 convolution is the fp32 accumulation:
+    1e-5 of the output's magnitude."""
+    from boostmvsnerfs_b200 import ops
+    from boostmvsnerfs_b200.mlp_pack import pack_conv3d_k3_umma
+    N, Cin, Cout, D, H, W = shape
+    g = torch.Generator(device="cuda").manual_seed(D + H)
+    xh = torch.randn((N, Cin, D, H, W), device="cuda", generator=g).half().contiguous(memory_format=torch.channels_last_3d)
+    w = (torch.randn((Cout, Cin, 3, 3, 3), device="cuda", generator=g) * 0.1).half().float()
+    b = torch.randn(Cout, device="cuda", generator=g)
+    out2 = torch.empty((N, 1, D, H, W), device="cuda")
+    feat = ops.conv3d_k3(xh, pack_conv3d_k3_umma(w), b, Cout, False, out2=out2, split=8, engine="umma")
+    got = torch.cat([feat, out2], dim=1).double()
+    ref = torch.nn.functional.conv3d(xh.double(), w.double(), b.double(), padding=1)
+    scale = ref.abs().max().item()
+    err = (got - ref).abs().max().item()
+    assert err <= 1e-5 * scale, (err, scale)
 
 
 # ------------------------------------------------------------------------------------------ FPN middle layers (conv2d_mma.cu)

@@ -37,11 +37,18 @@ def _setup(H, W, N, K, seed, smooth, depth_inv=False):
     return scene, depth, std, nf, vols, feat, rgb, cams, nerf, packed, triples
 
 
-@pytest.mark.parametrize("H,W,K,smooth,depth_inv", [(64, 96, 4, True, False), (64, 96, 1, False, False), (96, 160, 8, False, False),
-                                                    (64, 96, 3, True, True)])
-def test_multi_matches_per_chain_kernel(H, W, K, smooth, depth_inv):
+def _with_samples(cases):
+    """Every case at S = 1, 2, 3, 8 samples per ray.  S = 2 (the ENeRF configs, the kernels' `si >> 1` branch) keeps the
+    case's plain id; the others run the general `si / S` branch, and S = 3 makes rays straddle the 32-sample rounds
+    (mma) and the 128-sample tiles (tcgen05)."""
+    return [pytest.param(*c, S, id="-".join(map(str, c)) + ("" if S == 2 else f"-S{S}")) for c in cases for S in (1, 2, 3, 8)]
+
+
+@pytest.mark.parametrize("H,W,K,smooth,depth_inv,S", _with_samples([(64, 96, 4, True, False), (64, 96, 1, False, False),
+                                                                    (96, 160, 8, False, False), (64, 96, 3, True, True)]))
+def test_multi_matches_per_chain_kernel(H, W, K, smooth, depth_inv, S):
     from boostmvsnerfs_b200 import ops
-    N, S = 4, 2
+    N = 4
     scene, depth, std, nf, vols, feat, rgb, cams, nerf, packed, triples = _setup(H, W, N, K, 11 + K, smooth, depth_inv)
     rays = scene["rays_1"][0]
     multi = ops.render_rays_multi(depth, std, nf, rays, H, W, depth_inv, S, vols, feat, rgb, cams, triples, packed, want_count=True)
@@ -139,14 +146,17 @@ def test_network_uses_the_multi_launch_and_matches_per_chain(monkeypatch):
 
 
 # ------------------------------------------------------------------------------------------ tcgen05 engine
-@pytest.mark.parametrize("H,W,K,smooth,depth_inv", [(64, 96, 4, True, False), (64, 96, 1, False, False), (96, 160, 8, False, False),
-                                                    (64, 96, 3, True, True), (32, 40, 2, True, False)])
-def test_umma_engine_matches_the_mma_engine(H, W, K, smooth, depth_inv):
+@pytest.mark.parametrize("H,W,K,smooth,depth_inv,S", _with_samples([(64, 96, 4, True, False), (64, 96, 1, False, False),
+                                                                    (96, 160, 8, False, False), (64, 96, 3, True, True),
+                                                                    (32, 40, 2, True, False)]))
+def test_umma_engine_matches_the_mma_engine(H, W, K, smooth, depth_inv, S):
     """bmv_render_rays_multi_umma (MLP as tcgen05.mma, accumulators in tensor memory, two threads per sample row) against
     bmv_render_rays_multi: the gather is the same code (z / visibility bit-identical), the MLP the same hi / lo split
-    products in another summation order."""
+    products in another summation order.  Both engines against a ragged sub-range of their own launch, and at S = 3
+    against the stand-alone fetch followed by the NeRF module in float64."""
+    import copy
     from boostmvsnerfs_b200 import mlp_pack, ops
-    N, S = 4, 2
+    N = 4
     scene, depth, std, nf, vols, feat, rgb, cams, nerf, packed, triples = _setup(H, W, N, K, 11 + K, smooth, depth_inv)
     packed_u = mlp_pack.pack_nerf_weights_umma(nerf)
     rays = scene["rays_1"][0]
@@ -162,6 +172,26 @@ def test_umma_engine_matches_the_mma_engine(H, W, K, smooth, depth_inv):
     one = ops.render_rays(depth[0], std[0], nf[0], rays, H, W, depth_inv, S, vols[0], feat, rgb, cams, triples[0], packed_f, engine="fma")
     err = float((got["raw"][0] - one["raw"]).abs().max()) / float(one["raw"].abs().max())
     assert err <= (3e-5 if smooth else 2e-4), f"vs fp32 FMA kernel: {err:.2e}"
+    # ragged ray range: an odd first ray, and 1001 rays whose samples straddle rounds / tiles unless S divides 32
+    b, n = 37, 1001
+    for engine, full in (("mma", ref), ("umma", got)):
+        part = ops.render_rays_multi(depth, std, nf, rays, H, W, depth_inv, S, vols, feat, rgb, cams, triples,
+                                     packed if engine == "mma" else packed_u, ray_begin=b, n_rays=n, want_count=True)
+        for k_ in ("raw", "z_vals", "vis_mask", "vis_count"):
+            assert torch.equal(part[k_], full[k_][:, b:b + n]), f"{engine}: {k_} of rays [{b}, {b + n})"
+    if S != 3 or not smooth:
+        return
+    # independent reference for chain 0: the stand-alone K3 fetch (pinned to the golden vectors) + the NeRF module in float64
+    fetch = ops.raygen_sample_fetch(depth[0], std[0], nf[0], rays, H, W, depth_inv, S, vols[0], feat, rgb, cams, triples[0],
+                                    want=("z_vals", "vox_feat", "img_feat", "vis_mask"))
+    with torch.no_grad():
+        raw64 = copy.deepcopy(nerf).double()(fetch["vox_feat"].double()[None], fetch["img_feat"].double()[None])[0].view(-1, S, 4)
+    scale = float(raw64.abs().max())
+    for engine, res in (("mma", ref), ("umma", got)):
+        assert torch.equal(res["z_vals"][0], fetch["z_vals"]), f"{engine}: z vs the fetch"
+        assert torch.equal(res["vis_mask"][0], fetch["vis_mask"]), f"{engine}: visibility vs the fetch"
+        err = float((res["raw"][0].double() - raw64).abs().max()) / scale
+        assert err <= 2e-5, f"{engine}: raw differs from the float64 MLP by {err:.2e} of range"
 
 
 def test_umma_engine_device_views_ragged_range_generated_rays_and_replay():
@@ -187,3 +217,53 @@ def test_umma_engine_device_views_ragged_range_generated_rays_and_replay():
     g = ops.render_rays_multi(depth, std, nf, gen, H, W, False, S, vols, feat, rgb, cams, triples, packed_u)
     assert torch.equal(g["z_vals"], full["z_vals"]) and torch.equal(g["vis_mask"], full["vis_mask"])
     assert float((g["raw"] - full["raw"]).abs().max()) <= 1e-6
+
+
+# ------------------------------------------------------------------------------------------ row slabs (sharded frames)
+@pytest.mark.parametrize("H,W", [(64, 96), (66, 98)])
+@pytest.mark.parametrize("depth_inv", [False, True])
+@pytest.mark.parametrize("G", [2, 3, 4, 8])
+@pytest.mark.parametrize("engine", ["mma", "umma"])
+def test_row_slabs_match_the_full_grid(engine, G, depth_inv, H, W):
+    """Each rank of a G-way sharded frame renders the row tile dist.row_tile from the row slab dist.slab_rows of the
+    volumes and maps (ShardedFrameRenderer.render_tile: grid_rows, vol_row0, map_row0).  Every slab here sits between
+    NaN guard rows, above and below each plane, so a read outside it poisons the output instead of returning a
+    neighbour's finite data or vanishing under a zero weight: the tile must equal the slice of the full-grid launch bit
+    for bit.  Reading the volume or the maps one row off (vol_row0 or map_row0 = y0 + 1, still inside the guards) must
+    change the output."""
+    from boostmvsnerfs_b200 import dist, mlp_pack, ops
+    N, K, S, guard = 4, 3, 2, 2
+    scene, depth, std, nf, vols, feat, rgb, cams, nerf, packed, triples = _setup(H, W, N, K, 7 + G, True, depth_inv)
+    if engine == "umma":
+        packed = mlp_pack.pack_nerf_weights_umma(nerf)
+    _, hv, wv = depth.shape
+    D = vols.shape[2]
+    rays = ops.RayGenerator.from_cameras(scene["tar_ext"][0].cpu(), scene["tar_ixt"][0].cpu(), H, W, 1.0, "cuda")
+    full = ops.render_rays_multi(depth, std, nf, rays, H, W, depth_inv, S, vols, feat, rgb, cams, triples, packed,
+                                 want_count=True, engine=engine)
+    maps_full = torch.cat([depth[:, None], std[:, None], nf], dim=1)           # (K,4,hv,wv): [depth, std, near, far]
+    vol_full = vols.permute(0, 2, 3, 4, 1)                                     # (K,D,hv,wv,8) physical layout
+    nan = float("nan")
+    for q in range(G):
+        t0, t1 = dist.row_tile(H, G, q)
+        y0, y1 = dist.slab_rows(t0, t1, H, hv)
+        rows = y1 - y0
+        mbuf = torch.full((K, 4, rows + 2 * guard, wv), nan, device="cuda")
+        mbuf[:, :, guard:guard + rows] = maps_full[:, :, y0:y1]
+        maps = mbuf[:, :, guard:guard + rows]
+        vbuf = torch.full((K, D, rows + 2 * guard, wv, 8), nan, device="cuda")
+        vbuf[:, :, guard:guard + rows] = vol_full[:, :, y0:y1]
+        slab_vols = vbuf[:, :, guard:guard + rows].permute(0, 4, 1, 2, 3)      # (K,8,D,rows,wv) channels-last-3d
+        sl = slice(t0 * W, t1 * W)
+
+        def render(vol_row0, map_row0):
+            return ops.render_rays_multi(maps[:, 0], maps[:, 1], maps[:, 2:4], rays, H, W, depth_inv, S, slab_vols, feat, rgb,
+                                         cams, triples, packed, ray_begin=t0 * W, n_rays=(t1 - t0) * W, want_count=True,
+                                         grid_rows=hv, vol_row0=vol_row0, map_row0=map_row0, engine=engine)
+        got = render(y0, y0)
+        for k_ in ("raw", "z_vals", "vis_mask", "vis_count"):
+            assert torch.equal(got[k_], full[k_][:, sl]), (f"rank {q}/{G}: rows [{t0}, {t1}) from slab [{y0}, {y1}): {k_} "
+                                                          f"({int(got[k_].isnan().sum())} NaN)")
+        # the controls: one row off (never more than the guard depth) must show
+        assert not torch.equal(render(y0 + 1, y0)["raw"], full["raw"][:, sl]), f"rank {q}/{G}: a shifted volume slab went unnoticed"
+        assert not torch.equal(render(y0, y0 + 1)["z_vals"], full["z_vals"][:, sl]), f"rank {q}/{G}: shifted maps went unnoticed"
