@@ -11,6 +11,7 @@ LIB_PATH = os.path.join(HERE, "libbmv.so")
 
 MAX_VIEWS = 8
 MAX_VOLUMES = 16
+FRAME_SSIM_SCRATCH_WORDS = 2048
 
 f32p = C.POINTER(C.c_float)
 i32p = C.POINTER(C.c_int32)
@@ -206,6 +207,12 @@ class FrameToU8Params(C.Structure):
                 ("minmax_ord", C.c_void_p), ("minmax", C.c_void_p)]
 
 
+class FrameSsimParams(C.Structure):
+    _fields_ = [("pred", C.c_void_p), ("gt", C.c_void_p), ("H", i32), ("W", i32), ("crop_h", i32), ("crop_w", i32),
+                ("win_size", i32), ("reserved0", i32), ("data_range", C.c_double),
+                ("scratch", C.c_void_p), ("ssim", C.c_void_p)]
+
+
 ENTRY_POINTS = {
     "bmv_cost_volume_var": CostVolumeParams,
     "bmv_cost_volume_var_multi": CostVolumeMultiParams,
@@ -236,6 +243,7 @@ ENTRY_POINTS = {
     "bmv_conv3d_small": Conv3dSmallParams,
     "bmv_frame_psnr_accumulate": FramePsnrParams,
     "bmv_frame_to_u8": FrameToU8Params,
+    "bmv_frame_ssim": FrameSsimParams,
 }
 PLAIN_SYMBOLS = ("bmv_version", "bmv_last_error_string", "bmv_launch_count", "bmv_sizeof_params",
                  "bmv_nerf_mlp_weight_count", "bmv_render_rays_supported", "bmv_render_rays_mma_weight_words",

@@ -52,5 +52,6 @@ extern "C" BMV_API int bmv_sizeof_params(const char* entry) {
   if (!strcmp(entry, "bmv_render_rays_multi_umma")) return (int)sizeof(bmv_render_multi_params);
   if (!strcmp(entry, "bmv_frame_psnr_accumulate")) return (int)sizeof(bmv_frame_psnr_params);
   if (!strcmp(entry, "bmv_frame_to_u8")) return (int)sizeof(bmv_frame_to_u8_params);
+  if (!strcmp(entry, "bmv_frame_ssim")) return (int)sizeof(bmv_frame_ssim_params);
   return -1;
 }

@@ -1046,6 +1046,32 @@ def frame_psnr_accumulate(pred, gt, H, W, mask=None, crop=(0, 0), acc=None):
     return acc
 
 
+def frame_ssim(pred, gt, H, W, crop=(0, 0), win_size=7, data_range=2.0, out=None):
+    """SSIM of one frame, skimage.metrics.structural_similarity(gt, pred, channel_axis=-1, win_size=win_size,
+    data_range=data_range) with uniform weights, in float64 on the device (bmv_frame_ssim).  pred, gt: (H*W,3) fp32;
+    crop = (crop_h, crop_w) rows / columns dropped at each border before the metric sees the image.  Returns `out`, a
+    1-element float64 device tensor (allocated when None); nothing is read back.
+
+    The reference does not record the arguments its evaluator passes to skimage: the defaults are skimage's for a float
+    image (scikit-image <= 0.20: win_size 7, data_range 2 = the span of dtype_range[float32] = (-1, 1))."""
+    pred, gt = _cf32(pred.reshape(-1, 3), "pred"), _cf32(gt.reshape(-1, 3), "gt")
+    if pred.shape[0] != H * W or gt.shape[0] != H * W:
+        raise BmvError(f"frame_ssim: expected {H * W} pixels, got {pred.shape[0]} / {gt.shape[0]}")
+    if out is None:
+        out = torch.empty(1, device=pred.device, dtype=torch.float64)
+    elif not (torch.is_tensor(out) and out.is_cuda and out.dtype == torch.float64 and out.numel() == 1):
+        raise BmvError("frame_ssim: out must be a 1-element CUDA float64 tensor")
+    _on_current_device(out, "out")
+    scratch = torch.empty(_lib.FRAME_SSIM_SCRATCH_WORDS, device=pred.device, dtype=torch.float64)
+    p = _lib.FrameSsimParams()
+    p.pred, p.gt = pred.data_ptr(), gt.data_ptr()
+    p.H, p.W, p.crop_h, p.crop_w = H, W, int(crop[0]), int(crop[1])
+    p.win_size, p.data_range = int(win_size), float(data_range)
+    p.scratch, p.ssim = scratch.data_ptr(), out.data_ptr()
+    _lib.call("bmv_frame_ssim", p, _stream())
+    return out
+
+
 def frame_to_u8(rgb=None, depth=None):
     """rgb (R,3) fp32 -> uint8 `(rgb*255).astype(uint8)`; depth (R,) fp32 -> uint8 `((d-min)/(max-min)*255).astype(uint8)`
     (reference lib/visualizers/enerf.py:27-37).  Returns (rgb_u8 or None, depth_u8 or None, minmax (2,) fp32 or None)."""

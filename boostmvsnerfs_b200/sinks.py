@@ -2,12 +2,18 @@
 that touch every pixel of every frame, done on the device so that 4 instead of 16 bytes per pixel cross PCIe and the
 host never loops over a frame.
 
-  * `PsnrAccumulator.evaluate(output, batch)`  — reference lib/evaluators/enerf.py:37-71: per rendered level, the
-    prediction against `batch['rgb_{i}']` under `batch['msk_{i}']` (>= 1) and the optional 10 % centre crop
-    (`cfg.enerf.eval_center`), PSNR = 10 log10(1 / mse) as skimage.metrics.peak_signal_noise_ratio(data_range=1)
-    computes it (float64 mean of squared differences).  `summarize()` returns the mean over frames like
-    `Evaluator.summarize` (:104-106).  SSIM / LPIPS are library calls on the host in the reference (skimage, lpips) and
-    stay out of scope.
+  * `FrameEvaluator.evaluate(output, batch)`  — reference lib/evaluators/enerf.py:37-71: per rendered level, the
+    prediction against `batch['rgb_{i}']` (uploaded once for both metrics) with the optional 10 % centre crop
+    (`cfg.enerf.eval_center`):
+      - PSNR under `batch['msk_{i}']` (>= 1), = 10 log10(1 / mse) as skimage.metrics.peak_signal_noise_ratio(data_range=1)
+        computes it (float64 mean of squared differences);
+      - SSIM as skimage.metrics.structural_similarity(channel_axis=-1, win_size, data_range) computes it with uniform
+        weights (float64; no mask: skimage has none).  The reference does not record its SSIM arguments; the defaults
+        win_size=7, data_range=2.0 are skimage's for a float image.
+    Both stay on the device until `summarize()`, which reads them back and returns the means over frames of the last
+    level, {'psnr', 'ssim'}, like `Evaluator.summarize` (:104-106); `scene_psnrs` / `scene_ssims` hold every level per
+    scene.  `PsnrAccumulator` is its PSNR-only configuration.  LPIPS needs the VGG weights of the `lpips` package and
+    stays out of scope.
   * `FrameWriter.visualize(output, batch)` — reference lib/visualizers/enerf.py:21-37: uint8 colour image and
     min/max-normalised uint8 depth image of the last level; returned as host arrays (and written as binary PPM / PGM when
     `result_dir` is given; the reference writes JPEG through imageio, a host library that is not part of the path).
@@ -20,11 +26,13 @@ import torch
 from . import ops
 
 
-class PsnrAccumulator:
-    def __init__(self, rc, eval_center=False):
+class FrameEvaluator:
+    def __init__(self, rc, eval_center=False, ssim=True, win_size=7, data_range=2.0):
         self.rc, self.eval_center = rc, bool(eval_center)
-        self._pending = []            # (level, scene, device sse, device count): read back in summarize()
+        self.ssim, self.win_size, self.data_range = bool(ssim), int(win_size), float(data_range)
+        self._pending = []            # (level, scene, device (sse, count), device ssim or None): read back in summarize()
         self.psnrs, self.scene_psnrs = [], {}
+        self.ssims, self.scene_ssims = [], {}
 
     def evaluate(self, output, batch):
         rc = self.rc
@@ -40,21 +48,36 @@ class PsnrAccumulator:
                 msk = batch.get(f'msk_{i}')
                 m8 = None if msk is None else (msk[b].to(pred.device, non_blocking=True).reshape(-1) >= 1).to(torch.uint8)
                 acc = ops.frame_psnr_accumulate(pred, gt, h, w, mask=m8, crop=crop)
-                self._pending.append((i, batch['meta']['scene'][b], acc))
+                ssim = ops.frame_ssim(pred, gt, h, w, crop=crop, win_size=self.win_size,
+                                      data_range=self.data_range) if self.ssim else None
+                self._pending.append((i, batch['meta']['scene'][b], acc, ssim))
 
     def _drain(self):
-        for i, scene, (sse, cnt) in self._pending:
+        for i, scene, (sse, cnt), ssim in self._pending:
             n = int(cnt.item())
             mse = float(sse.item()) / n if n else float('nan')
             psnr = 10.0 * math.log10(1.0 / mse) if mse > 0 else float('inf')
             if i == self.rc.num - 1:
                 self.psnrs.append(psnr)
             self.scene_psnrs.setdefault(f'{scene}_level{i}', []).append(psnr)
+            if ssim is not None:
+                ssim = float(ssim.item())
+                if i == self.rc.num - 1:
+                    self.ssims.append(ssim)
+                self.scene_ssims.setdefault(f'{scene}_level{i}', []).append(ssim)
         self._pending = []
 
     def summarize(self):
         self._drain()
-        return {'psnr': sum(self.psnrs) / len(self.psnrs) if self.psnrs else float('nan')}
+        out = {'psnr': sum(self.psnrs) / len(self.psnrs) if self.psnrs else float('nan')}
+        if self.ssim:
+            out['ssim'] = sum(self.ssims) / len(self.ssims) if self.ssims else float('nan')
+        return out
+
+
+class PsnrAccumulator(FrameEvaluator):
+    def __init__(self, rc, eval_center=False):
+        super().__init__(rc, eval_center, ssim=False)
 
 
 class FrameWriter:

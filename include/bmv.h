@@ -609,7 +609,18 @@ BMV_API int bmv_render_rays_multi_umma(const bmv_render_multi_params* p, bmv_str
  * bmv_frame_to_u8: reference lib/visualizers/enerf.py:27-37 — rgb_u8 = (rgb * 255).astype(uint8);
  *   depth_u8 = ((depth - min) / (max - min) * 255).astype(uint8), min / max over the frame written to minmax[0..1]
  *   (optional).  minmax_ord: 2 words of device scratch.
+ * bmv_frame_ssim: the SSIM the reference's evaluator takes from skimage, structural_similarity(gt, pred,
+ *   channel_axis=-1, win_size, data_range) with uniform weights (scikit-image 0.19 / 0.20).  pred / gt (H*W,3) fp32
+ *   row-major, optional centre crop as above (the metric then sees only the cropped image).  Per channel: box means
+ *   ux, uy, uxx, uyy, uxy over the win_size x win_size window, v = w²/(w²-1) * (second moment - product of means),
+ *   S = (2 ux uy + C1)(2 vxy + C2) / ((ux² + uy² + C1)(vx + vy + C2)), C1 = (0.01 R)², C2 = (0.03 R)², averaged over
+ *   the pixels whose window lies inside the image; *ssim = mean of the three channel values.  All in float64.
+ *   win_size odd, >= 3 and <= both cropped sides; data_range > 0.  The reference does not record its arguments:
+ *   skimage's defaults for a float image are win_size 7 and data_range 2 (dtype range (-1, 1)).
+ *   scratch: BMV_FRAME_SSIM_SCRATCH_WORDS doubles of device scratch (per-CTA partials, summed in a fixed order: two
+ *   launches on the same inputs give the same bits).
  */
+#define BMV_FRAME_SSIM_SCRATCH_WORDS 2048
 typedef struct bmv_frame_psnr_params {
   const float* pred; const float* gt; const uint8_t* mask;   /* mask may be NULL */
   int32_t H, W, crop_h, crop_w;
@@ -624,6 +635,16 @@ typedef struct bmv_frame_to_u8_params {
   uint32_t* minmax_ord; float* minmax;      /* scratch (2 words); optional output (2 floats) */
 } bmv_frame_to_u8_params;
 BMV_API int bmv_frame_to_u8(const bmv_frame_to_u8_params* p, bmv_stream_t stream);
+
+typedef struct bmv_frame_ssim_params {
+  const float* pred; const float* gt;
+  int32_t H, W, crop_h, crop_w;
+  int32_t win_size, reserved0;
+  double data_range;
+  double* scratch;                          /* DEVICE, BMV_FRAME_SSIM_SCRATCH_WORDS doubles */
+  double* ssim;                             /* DEVICE, 1 double: the frame's SSIM */
+} bmv_frame_ssim_params;
+BMV_API int bmv_frame_ssim(const bmv_frame_ssim_params* p, bmv_stream_t stream);
 
 #ifdef __cplusplus
 }
