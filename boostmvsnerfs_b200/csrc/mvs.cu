@@ -396,6 +396,9 @@ extern "C" BMV_API int bmv_mvs_march_fetch(const bmv_mvs_march_params* p, bmv_st
   if (p->n_rays == 0) return BMV_OK;
   BMV_REQUIRE(p->rays && p->t && p->src_exts && p->src_ixts, BMV_ERR_INVALID_ARGUMENT, "bmv_mvs_march_fetch: null input");
   BMV_REQUIRE(p->V == 3, BMV_ERR_UNSUPPORTED_SHAPE, "bmv_mvs_march_fetch: V=%d views not instantiated (3)", p->V);
+  // a ray is read as two float4, and the staged 86-float rows are stored as float2
+  BMV_REQUIRE(((uintptr_t)p->rays & 15) == 0 && ((uintptr_t)p->mlp_in & 7) == 0, BMV_ERR_INVALID_ARGUMENT,
+              "bmv_mvs_march_fetch: rays must be 16-byte aligned and mlp_in 8-byte aligned");
   if (p->mlp_in)
     BMV_REQUIRE(p->volume && p->rgb && p->Cv == 8 && p->Dv >= 1 && p->hv >= 1 && p->wv >= 1 && p->H >= 2 && p->W >= 2,
                 BMV_ERR_INVALID_ARGUMENT, "bmv_mvs_march_fetch: volume/rgb inputs missing or Cv != 8");

@@ -515,6 +515,8 @@ extern "C" BMV_API int bmv_mvs_render_umma(const bmv_mvs_render_params* rp, bmv_
   BMV_REQUIRE(p->Dv >= 1 && p->hv >= 1 && p->wv >= 1 && p->H >= 2 && p->W >= 2, BMV_ERR_INVALID_ARGUMENT, "bmv_mvs_render_umma: bad grid size");
   BMV_REQUIRE(((uintptr_t)rp->weights & 15) == 0 && ((uintptr_t)rp->raw & 15) == 0 && ((uintptr_t)p->rays & 15) == 0,
               BMV_ERR_INVALID_ARGUMENT, "bmv_mvs_render_umma: weights / raw / rays must be 16-byte aligned");
+  BMV_REQUIRE(!p->rgb_nhwc4 || ((uintptr_t)p->rgb & 15) == 0, BMV_ERR_INVALID_ARGUMENT,
+              "bmv_mvs_render_umma: an (N,H,W,4) rgb image must be 16-byte aligned");
   BMV_REQUIRE(p->vol_c_stride != 1 || (((uintptr_t)p->volume & 15) == 0 && p->vol_x_stride % 4 == 0 && p->vol_y_stride % 4 == 0 &&
                                        p->vol_d_stride % 4 == 0),
               BMV_ERR_INVALID_ARGUMENT, "bmv_mvs_render_umma: a channels-last volume must have 16-byte aligned voxels");

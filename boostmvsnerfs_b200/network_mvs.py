@@ -169,24 +169,27 @@ class BoostMvsnerfNetwork(nn.Module):
         """reference lib/networks/boost_mvsnerf/network.py:23-95: for every triple of source views march
         128 uniform samples, volume-render the visibility score into a 2-D coverage mask, then pick the
         K triples greedily by newly covered area.  All on the GPU, no network involved."""
+        picked = greedy_coverage(self.view_selection_masks(batch), self.rc.k_best)
+        key = f"{batch['meta']['scene'][0]}_{batch['meta']['tar_view'][0]}"
+        return {key: picked}
+
+    def view_selection_masks(self, batch):
+        """The 2-D coverage mask of every triple of source views (reference calc_mask,
+        lib/networks/boost_mvsnerf/network.py:23-45), in the order of itertools.combinations -> (T, 1, R)."""
         self._check(batch)
-        rc = self.rc
         N = batch['all_src_inps'].shape[1]
         H, W = batch['all_src_inps'].shape[-2:]
-        table = list(itertools.combinations(range(N), 3))
         rays = batch['rays_0'][0]
         S = 128
         masks = []
         with torch.no_grad():
-            for tr in table:
+            for tr in itertools.combinations(range(N), 3):
                 o = ops.mvs_march_fetch(rays, S, tr, batch['all_src_exts'][0], batch['all_src_ixts'][0], H, W,
                                         0.0, 1.0, None, None, want=("z_vals", "vis_mask"))
                 m = (o['vis_mask'] / S).unsqueeze(-1).expand(-1, -1, 4).contiguous()
-                rgbm, _, _ = ops.composite(m, o['z_vals'], rc.white_bkgd)
+                rgbm, _, _ = ops.composite(m, o['z_vals'], self.rc.white_bkgd)
                 masks.append(rgbm.mean(-1)[None])                         # (1,R)
-            picked = greedy_coverage(torch.stack(masks), rc.k_best)
-        key = f"{batch['meta']['scene'][0]}_{batch['meta']['tar_view'][0]}"
-        return {key: picked}
+        return torch.stack(masks)
 
 
 def greedy_coverage(masks, k):

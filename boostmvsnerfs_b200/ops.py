@@ -723,6 +723,8 @@ def mvs_march_fetch(rays, S, views, src_exts, src_ixts, H, W, near, far, volume,
     dev = rays.device
     R = rays.shape[0]
     n = R - ray_begin if n_rays is None else n_rays
+    if not (0 <= ray_begin and 0 <= n and ray_begin + n <= R):
+        raise BmvError(f"mvs_march_fetch: rays [{ray_begin}, {ray_begin + n}) outside the {R} rays given")
     p = _lib.MvsMarchParams()
     p.rays, p.ray_begin, p.n_rays = rays.data_ptr(), ray_begin, n
     t = _linspace(S, dev)
@@ -1215,6 +1217,8 @@ def mvs_render(rays, S, views, src_exts, src_ixts, H, W, near, far, volume, rgb,
     dev = rays.device
     R = rays.shape[0]
     n = R - ray_begin if n_rays is None else n_rays
+    if not (0 <= ray_begin and 0 <= n and ray_begin + n <= R):
+        raise BmvError(f"mvs_render: rays [{ray_begin}, {ray_begin + n}) outside the {R} rays given")
     w = packed_weights
     if not (torch.is_tensor(w) and w.is_cuda and w.dtype == torch.int32 and w.is_contiguous()
             and w.numel() * 4 == _lib.load().bmv_mvs_render_umma_weight_bytes()):
