@@ -31,11 +31,26 @@
 // accumulation — the same split as render_mma.cu / render_multi.cu, so raw agrees with the fp32 kernels to ~1e-5; z and
 // visibility are bit-identical to render_multi.cu (same code).
 //
-// Shared memory: packed weights (mlp_pack.pack_nerf_weights_umma, nerf_umma_pack.cuh) + two operand tiles of 20 K-chunks
-// (chunk = 128 rows x 16 B hi slab + the same for lo; UMMA K-major SWIZZLE_NONE: SBO = 128 B, LBO = 4096 B):
-//   0,1 var | 2,3 mean | 4+2v,5+2v x_v   (phase A; later 0..3 = im, 0..7 = hid)      10+2v,11+2v f_v = [feat8 | rgb3 dir4 0]
-//   16,17 pooled (before that: the phase-B exchange)      18 vox      19 (1, 0, ...): bias column of lr0 / color.0
-// TMEM (512 columns, 256 per tile): G_v 32v | fc 96 | lr0 112..175 ; then colour: shared 0..63, per view 64 + 64v.
+// Operands.  The A operands of phases 0..2 (global_fc, agg.fc, lr0: 13 of the 22 K-steps) go to tensor memory with
+// tcgen05.st and the MMAs read them from there (the TS form; only the weights come from shared memory): the rows come
+// out of TMEM (tcgen05.ld) into registers for ReLU / soft-max anyway, and st.shared + the tensor core's shared-memory
+// reads of A were the largest shared-memory traffic of a tile.  Phase 3 (color.0, 27 MMAs) keeps A in shared memory:
+// its accumulators fill all 256 TMEM columns of the tile (shared 64 + 3 views x 64), and its A operands (hid, pooled,
+// vox | 1, f_v) would need another 224.  Measured (profiles/round4_render_tmem_operands.md, B200 at 1000 W): 1.497 ->
+// 1.347 ms for the 4 chains of the C2 frame, bit-identical raw.
+// Shared memory: packed weights (mlp_pack.pack_nerf_weights_umma, nerf_umma_pack.cuh) + two operand tiles of 18 K-chunks
+// (chunk = 128 rows x 16 B hi slab + the same for lo; UMMA K-major SWIZZLE_NONE: SBO = 128 B, LBO = 4096 B), all A of color.0:
+//   0..7 hid      8+2v,9+2v f_v = [feat8 | rgb3 dir4 0]      14,15 pooled (before that: the phase-B exchange)
+//   16 vox      17 (1, 0, ...): bias column of color.0
+// TMEM (512 columns, 256 per tile; an A slab = one K = 16 step = hi 8 columns + lo 8 columns, two fp16 per column):
+//   phase 0: G_v 32v (accumulators) | A: var 96, mean 112, x_v 128 + 16v, [vox | 1 0 ...] 176..191 (bias column of lr0)
+//   phase 1: A: im 96..127 (over var, mean) | fc 128..143 (over x_0)
+//   phase 2: A: pooled 96..111 (over im), [vox | 1] 176 | lr0 112..175
+//   phase 3: colour: shared 0..63, per view 64 + 64v (A in shared memory)
+// Each reused column range was last read by an MMA that has completed (the epilogue waited on its commit) or by
+// tcgen05.ld of all 8 warps (retired before they arrive on `ready`).  The exception is the next unit's operand slabs
+// over the colour accumulators: the half-0 warp stores its slabs right after phase E's pair barrier, so the half-1
+// warp of the same lane quarter retires its tcgen05.ld of those columns before that barrier.
 #include <stdlib.h>
 
 #include "lean_gather.cuh"
@@ -47,39 +62,58 @@
 namespace bmv {
 
 constexpr int RU_CHUNK = 4096, RU_LO = 2048;               // bytes per K-chunk (hi slab + lo slab), offset of the lo slab
-constexpr int RU_VAR = 0, RU_MEAN = 2, RU_X = 4, RU_IM = 0, RU_HID = 0, RU_F = 10, RU_POOLED = 16, RU_VOX = 18, RU_ONE = 19;
-constexpr int RU_TILE_BYTES = 20 * RU_CHUNK;               // 81920
+constexpr int RU_HID = 0, RU_F = 8, RU_POOLED = 14, RU_VOX = 16, RU_ONE = 17;
+constexpr int RU_TILE_BYTES = 18 * RU_CHUNK;               // 73728
 constexpr int RU_ROW_WARPS = 16;
 constexpr int RU_THREADS = RU_ROW_WARPS * 32;
 constexpr int RU_PACK_PADDED = (UMMA_PACK_BYTES + 127) / 128 * 128;
 constexpr size_t RU_SMEM = (size_t)RU_PACK_PADDED + 2 * (size_t)RU_TILE_BYTES + 128;
-constexpr int RU_T_G = 0, RU_T_FC = 96, RU_T_L0 = 112, RU_T_CS = 0, RU_T_CV = 64;   // TMEM columns within a tile's 256
+// TMEM columns within a tile's 256: accumulators and the A slabs of phases 0..2 (16 columns each: hi 8 + lo 8)
+constexpr int RU_T_G = 0, RU_T_VAR = 96, RU_T_MEAN = 112, RU_T_X = 128, RU_T_VOX = 176;            // phase 0
+constexpr int RU_T_IM = 96, RU_T_FC = 128, RU_T_POOLED = 96, RU_T_L0 = 112, RU_T_CS = 0, RU_T_CV = 64;
 
-// this row's 8 values of K-chunk `chunk`: 16 B into the hi slab, 16 B into the lo slab
-__device__ __forceinline__ void ru_put(unsigned char* tile, int chunk, int row, float v0, float v1, float v2, float v3, float v4,
-                                       float v5, float v6, float v7) {
-  uint4 hi, lo;
-  split_pack(v0, v1, hi.x, lo.x); split_pack(v2, v3, hi.y, lo.y); split_pack(v4, v5, hi.z, lo.z); split_pack(v6, v7, hi.w, lo.w);
+// this row's 8 values of one K-chunk as fp16 hi / lo pairs
+struct RuWords {
+  uint32_t hi[4], lo[4];
+};
+__device__ __forceinline__ RuWords ru_split(float v0, float v1, float v2, float v3, float v4, float v5, float v6, float v7) {
+  RuWords w;
+  split_pack(v0, v1, w.hi[0], w.lo[0]); split_pack(v2, v3, w.hi[1], w.lo[1]);
+  split_pack(v4, v5, w.hi[2], w.lo[2]); split_pack(v6, v7, w.hi[3], w.lo[3]);
+  return w;
+}
+__device__ __forceinline__ RuWords ru_split(const float* v) { return ru_split(v[0], v[1], v[2], v[3], v[4], v[5], v[6], v[7]); }
+// shared-memory K-chunk `chunk`: 16 B into the hi slab, 16 B into the lo slab
+__device__ __forceinline__ void ru_put(unsigned char* tile, int chunk, int row, const RuWords& w) {
   unsigned char* q = tile + chunk * RU_CHUNK + row * 16;
-  *reinterpret_cast<uint4*>(q) = hi;
-  *reinterpret_cast<uint4*>(q + RU_LO) = lo;
+  *reinterpret_cast<uint4*>(q) = make_uint4(w.hi[0], w.hi[1], w.hi[2], w.hi[3]);
+  *reinterpret_cast<uint4*>(q + RU_LO) = make_uint4(w.lo[0], w.lo[1], w.lo[2], w.lo[3]);
 }
-__device__ __forceinline__ void ru_put(unsigned char* tile, int chunk, int row, const float* v) {
-  ru_put(tile, chunk, row, v[0], v[1], v[2], v[3], v[4], v[5], v[6], v[7]);
+// TMEM: K-chunk j (0 | 1) of the slab at column c is taddr = c + 4 j: hi words there, lo words 8 columns further
+__device__ __forceinline__ void ru_put_tm(uint32_t taddr, const RuWords& w) {
+  tmem_st4(taddr, w.hi);
+  tmem_st4(taddr + 8, w.lo);
 }
 
-// one K = 16 step of a split product: D (+)= A_lo B_hi + A_hi B_lo + A_hi B_hi; a / b: descriptor low words of the hi
-// operands (start address >> 4 | LBO field), the lo slab / block a constant further
-template <bool ACC>
+// one K = 16 step of a split product: D (+)= A_lo B_hi + A_hi B_lo + A_hi B_hi; a: TMEM address of the A slab (hi
+// columns, lo 8 further) or descriptor low word of the shared hi operand (lo a chunk's lo offset further); b: descriptor
+// low word of the hi weights (start address >> 4 | LBO field), the lo block a constant further
+template <bool ACC, bool A_TMEM>
 __device__ __forceinline__ void ru_kstep(uint32_t d, uint32_t a, uint32_t b, uint32_t idesc) {
   constexpr uint32_t HI = (128u >> 4) | (1u << 14);        // SBO = 128 B, descriptor version 1, SWIZZLE_NONE
-  umma_f16_lohi<ACC>(d, a + (RU_LO >> 4), HI, b, HI, idesc);
-  umma_f16_lohi<true>(d, a, HI, b + (UW_BLOCK >> 4), HI, idesc);
-  umma_f16_lohi<true>(d, a, HI, b, HI, idesc);
+  if constexpr (A_TMEM) {
+    umma_f16_ts<ACC>(d, a + 8, b, HI, idesc);
+    umma_f16_ts<true>(d, a, b + (UW_BLOCK >> 4), HI, idesc);
+    umma_f16_ts<true>(d, a, b, HI, idesc);
+  } else {
+    umma_f16_lohi<ACC>(d, a + (RU_LO >> 4), HI, b, HI, idesc);
+    umma_f16_lohi<true>(d, a, HI, b + (UW_BLOCK >> 4), HI, idesc);
+    umma_f16_lohi<true>(d, a, HI, b, HI, idesc);
+  }
 }
 
 // every tcgen05.mma of one phase of one tile (executed by one elected lane); acc: the tile's TMEM base, a: descriptor low
-// word of the tile's chunk 0, wB: shared-memory address of the packed weights
+// word of the tile's shared chunk 0, wB: shared-memory address of the packed weights
 template <int PHASE>
 __device__ __forceinline__ void ru_issue_phase(uint32_t acc, uint32_t a, uint32_t wB) {
   constexpr uint32_t CH = RU_CHUNK >> 4;                   // one K-chunk in descriptor address units
@@ -89,27 +123,27 @@ __device__ __forceinline__ void ru_issue_phase(uint32_t acc, uint32_t a, uint32_
 #pragma unroll
     for (int v = 0; v < 3; ++v) {
       const uint32_t d = acc + RU_T_G + 32 * v;
-      ru_kstep<false>(d, a + RU_VAR * CH, bGS, id);
-      ru_kstep<true>(d, a + RU_MEAN * CH, bGS + 2 * 32, id);
-      ru_kstep<true>(d, a + (RU_X + 2 * v) * CH, bGV, id);
+      ru_kstep<false, true>(d, acc + RU_T_VAR, bGS, id);
+      ru_kstep<true, true>(d, acc + RU_T_MEAN, bGS + 2 * 32, id);
+      ru_kstep<true, true>(d, acc + RU_T_X + 16 * v, bGV, id);
     }
   } else if constexpr (PHASE == 1) {                       // agg.fc: im (K = 32) -> 16
     const uint32_t id = umma_idesc(16), bFC = desc_lo(wB + UW_FC, 16 * 16);
-    ru_kstep<false>(acc + RU_T_FC, a + RU_IM * CH, bFC, id);
-    ru_kstep<true>(acc + RU_T_FC, a + (RU_IM + 2) * CH, bFC + 2 * 16, id);
+    ru_kstep<false, true>(acc + RU_T_FC, acc + RU_T_IM, bFC, id);
+    ru_kstep<true, true>(acc + RU_T_FC, acc + RU_T_IM + 16, bFC + 2 * 16, id);
   } else if constexpr (PHASE == 2) {                       // lr0: [pooled | vox 1] (K = 32) -> 64
     const uint32_t id = umma_idesc(64), bL0 = desc_lo(wB + UW_L0, 64 * 16);
-    ru_kstep<false>(acc + RU_T_L0, a + RU_POOLED * CH, bL0, id);
-    ru_kstep<true>(acc + RU_T_L0, a + RU_VOX * CH, bL0 + 2 * 64, id);
+    ru_kstep<false, true>(acc + RU_T_L0, acc + RU_T_POOLED, bL0, id);
+    ru_kstep<true, true>(acc + RU_T_L0, acc + RU_T_VOX, bL0 + 2 * 64, id);
   } else {                                                 // color.0: shared part once, per-view parts next to it
     const uint32_t id = umma_idesc(64), bCS = desc_lo(wB + UW_CS, 64 * 16), bCV = desc_lo(wB + UW_CV, 64 * 16);
-    ru_kstep<false>(acc + RU_T_CS, a + RU_HID * CH, bCS, id);
+    ru_kstep<false, false>(acc + RU_T_CS, a + RU_HID * CH, bCS, id);
 #pragma unroll
-    for (int ks = 1; ks < 4; ++ks) ru_kstep<true>(acc + RU_T_CS, a + (RU_HID + 2 * ks) * CH, bCS + ks * 2 * 64, id);
-    ru_kstep<true>(acc + RU_T_CS, a + RU_POOLED * CH, bCS + 4 * 2 * 64, id);
-    ru_kstep<true>(acc + RU_T_CS, a + RU_VOX * CH, bCS + 5 * 2 * 64, id);
+    for (int ks = 1; ks < 4; ++ks) ru_kstep<true, false>(acc + RU_T_CS, a + (RU_HID + 2 * ks) * CH, bCS + ks * 2 * 64, id);
+    ru_kstep<true, false>(acc + RU_T_CS, a + RU_POOLED * CH, bCS + 4 * 2 * 64, id);
+    ru_kstep<true, false>(acc + RU_T_CS, a + RU_VOX * CH, bCS + 5 * 2 * 64, id);
 #pragma unroll
-    for (int v = 0; v < 3; ++v) ru_kstep<false>(acc + RU_T_CV + 64 * v, a + (RU_F + 2 * v) * CH, bCV, id);
+    for (int v = 0; v < 3; ++v) ru_kstep<false, false>(acc + RU_T_CV + 64 * v, a + (RU_F + 2 * v) * CH, bCV, id);
   }
 }
 
@@ -120,7 +154,8 @@ __device__ __forceinline__ void ru_issue_phase(uint32_t acc, uint32_t a, uint32_
 template <int PHASE>
 __device__ __forceinline__ void ru_publish_and_issue(uint32_t* cnt, uint32_t mb_ready, uint32_t& par_ready, uint32_t mb_acc, uint32_t acc,
                                                      uint32_t a, uint32_t wB, bool no_mma, int lane) {
-  proxy_fence_async();                 // generic-proxy st.shared -> visible to the tensor core (async proxy)
+  if constexpr (PHASE < 3) tmem_wait_st();    // this phase's A slabs (tcgen05.st) complete
+  if constexpr (PHASE != 1) proxy_fence_async();   // st.shared of phase 3's operands -> visible to the tensor core (async proxy)
   tc_fence_before();
   mbar_arrive(mb_ready);
   __syncwarp();
@@ -203,12 +238,10 @@ __global__ void __launch_bounds__(RU_THREADS, 1) render_multi_umma_kernel(bmv_re
     const uint32_t a_lo = ((smem_u32(tile) & 0x3FFFFu) >> 4) | ((uint32_t)(RU_CHUNK >> 4) << 16), wB = smem_u32(sW);
     const bool no_mma = dbg & 2;
     const int pair_bar = 1 + tile_id * 4 + wq;             // named barrier of the two warps that share this lane quarter
-    float4* xb_mine = reinterpret_cast<float4*>(tile + RU_POOLED * RU_CHUNK + half * RU_LO + row * 16);
-    const float4* xb_other = reinterpret_cast<const float4*>(tile + RU_POOLED * RU_CHUNK + (half ^ 1) * RU_LO + row * 16);
+    float4* xb = reinterpret_cast<float4*>(tile + RU_POOLED * RU_CHUNK + row * 16);   // phase-B exchange, + half * RU_LO
     const RmCtx c = lean_ctx(p, mp.nf_plane_stride);
     const bool unit_scale = p.render_scale == 1.f;
     const int vol_row0 = mp.vol_row0, map_row0 = mp.map_row0;
-    const float ba = sV[UV_SC], bs = sV[UV_SC + 1], b2 = sV[UV_SC + 2];
     const bool skip_gather = dbg & 1, skip_epi = dbg & 4;
     uint32_t par_acc = 0;
     bool first = true;
@@ -243,14 +276,13 @@ __global__ void __launch_bounds__(RU_THREADS, 1) render_multi_umma_kernel(bmv_re
             float f[8], d[4];
             lean_fetch_feat(p, view, tp, f);
             lean_dir_feat(cam, q, tt, d);
-            ru_put(tile, RU_F + 2 * v, row, f);
+            ru_put(tile, RU_F + 2 * v, row, ru_split(f));
 #pragma unroll
             for (int ch = 0; ch < 8; ++ch) {
               const float4 w = *reinterpret_cast<const float4*>(sV + UV_WV + ch * 4);
               const float e = fmaf(w.w, d[3], fmaf(w.z, d[2], fmaf(w.y, d[1], fmaf(w.x, d[0], sV[UV_BV + ch]))));
               x[v][ch] = f[ch] + fmaxf(e, 0.f);
             }
-            ru_put(tile, RU_X + 2 * v, row, x[v]);
           }
           float var[8], mean[8];
 #pragma unroll
@@ -260,8 +292,11 @@ __global__ void __launch_bounds__(RU_THREADS, 1) render_multi_umma_kernel(bmv_re
             mean[ch] = m;
             var[ch] = fmaf(e2, e2, fmaf(e1, e1, e0 * e0)) * 0.5f;
           }
-          ru_put(tile, RU_VAR, row, var);
-          ru_put(tile, RU_MEAN, row, mean);
+          __syncwarp();                                    // tcgen05.st is warp-collective
+#pragma unroll
+          for (int v = 0; v < V; ++v) ru_put_tm(tcol + RU_T_X + 16 * v, ru_split(x[v]));
+          ru_put_tm(tcol + RU_T_VAR, ru_split(var));
+          ru_put_tm(tcol + RU_T_MEAN, ru_split(mean));
           if (live) {
             const int64_t oi = out0 + si;
             if (mp.z_vals) mp.z_vals[oi] = q.z;
@@ -270,10 +305,12 @@ __global__ void __launch_bounds__(RU_THREADS, 1) render_multi_umma_kernel(bmv_re
           }
         } else {
           // trilinear volume fetch; colours (channels 8..10) and direction features of the views
+          RuWords vox;
           {
-            float vox[8];
-            lean_vox_fetch(p, c, mp.volume + (int64_t)k * mp.vol_k_stride, vol_row0, q, vox);
-            ru_put(tile, RU_VOX, row, vox);
+            float vf[8];
+            lean_vox_fetch(p, c, mp.volume + (int64_t)k * mp.vol_k_stride, vol_row0, q, vf);
+            vox = ru_split(vf);
+            ru_put(tile, RU_VOX, row, vox);                // phase 3 reads vox from shared memory, phase 2 from TMEM
           }
           float x[V][3];
 #pragma unroll
@@ -284,14 +321,13 @@ __global__ void __launch_bounds__(RU_THREADS, 1) render_multi_umma_kernel(bmv_re
             float d[4];
             lean_fetch_rgb(p, view, tp, rgbv[v]);
             lean_dir_feat(cam, q, tt, d);
-            ru_put(tile, RU_F + 2 * v + 1, row, rgbv[v][0], rgbv[v][1], rgbv[v][2], d[0], d[1], d[2], d[3], 0.f);
+            ru_put(tile, RU_F + 2 * v + 1, row, ru_split(rgbv[v][0], rgbv[v][1], rgbv[v][2], d[0], d[1], d[2], d[3], 0.f));
 #pragma unroll
             for (int ch = 0; ch < 3; ++ch) {
               const float4 w = *reinterpret_cast<const float4*>(sV + UV_WV + (8 + ch) * 4);
               const float e = fmaf(w.w, d[3], fmaf(w.z, d[2], fmaf(w.y, d[1], fmaf(w.x, d[0], sV[UV_BV + 8 + ch]))));
               x[v][ch] = rgbv[v][ch] + fmaxf(e, 0.f);
             }
-            ru_put(tile, RU_X + 2 * v + 1, row, x[v][0], x[v][1], x[v][2], 0.f, 0.f, 0.f, 0.f, 0.f);
           }
           float var[3], mean[3];
 #pragma unroll
@@ -301,8 +337,15 @@ __global__ void __launch_bounds__(RU_THREADS, 1) render_multi_umma_kernel(bmv_re
             mean[ch] = m;
             var[ch] = fmaf(e2, e2, fmaf(e1, e1, e0 * e0)) * 0.5f;
           }
-          ru_put(tile, RU_VAR + 1, row, var[0], var[1], var[2], 0.f, 0.f, 0.f, 0.f, 1.f);   // K index 15: global_fc bias column
-          ru_put(tile, RU_MEAN + 1, row, mean[0], mean[1], mean[2], 0.f, 0.f, 0.f, 0.f, 0.f);
+          __syncwarp();                                    // tcgen05.st is warp-collective
+#pragma unroll
+          for (int v = 0; v < V; ++v) ru_put_tm(tcol + RU_T_X + 16 * v + 4, ru_split(x[v][0], x[v][1], x[v][2], 0.f, 0.f, 0.f, 0.f, 0.f));
+          ru_put_tm(tcol + RU_T_VAR + 4, ru_split(var[0], var[1], var[2], 0.f, 0.f, 0.f, 0.f, 1.f));   // K index 15: global_fc bias column
+          ru_put_tm(tcol + RU_T_MEAN + 4, ru_split(mean[0], mean[1], mean[2], 0.f, 0.f, 0.f, 0.f, 0.f));
+          // the whole [vox | 1 0 ... 0] slab of lr0 (K index 24: its bias column); phase 3 overwrites these columns
+          const uint32_t vs[16] = {vox.hi[0], vox.hi[1], vox.hi[2], vox.hi[3], 0x00003C00u, 0u, 0u, 0u,
+                                   vox.lo[0], vox.lo[1], vox.lo[2], vox.lo[3], 0u, 0u, 0u, 0u};
+          tmem_st16(tcol + RU_T_VOX, vs);
         }
       } else {
 #pragma unroll
@@ -330,9 +373,10 @@ __global__ void __launch_bounds__(RU_THREADS, 1) render_multi_umma_kernel(bmv_re
           }
           pl[v] = (a0 + a1) + (a2 + a3);
         }
-        *xb_mine = make_float4(pl[0], pl[1], pl[2], 0.f);
+        xb[half * (RU_LO / 16)] = make_float4(pl[0], pl[1], pl[2], 0.f);
         bar_sync_named(pair_bar, 64);
-        const float4 po = *xb_other;
+        const float4 po = xb[(half ^ 1) * (RU_LO / 16)];
+        const float ba = sV[UV_SC];                        // bias scalars are read where used: fewer live registers
         // both halves add (columns 0..15) + (columns 16..31) in this order: identical soft-max weights in both
         const float l0 = fmaxf((half ? po.x + pl[0] : pl[0] + po.x) + ba, 0.f);
         const float l1 = fmaxf((half ? po.y + pl[1] : pl[1] + po.y) + ba, 0.f);
@@ -344,8 +388,10 @@ __global__ void __launch_bounds__(RU_THREADS, 1) render_multi_umma_kernel(bmv_re
         float im[16];
 #pragma unroll
         for (int j = 0; j < 16; ++j) im[j] = fmaf(w2, g[2][j], fmaf(w1, g[1][j], w0 * g[0][j]));
-        ru_put(tile, RU_IM + 2 * half, row, im);
-        ru_put(tile, RU_IM + 2 * half + 1, row, im + 8);
+        uint32_t s[16];                                    // this half's K = 16 slab of agg.fc: hi 8 columns, lo 8
+#pragma unroll
+        for (int j = 0; j < 8; ++j) split_pack(im[2 * j], im[2 * j + 1], s[j], s[8 + j]);
+        tmem_st16(tcol + RU_T_IM + 16 * half, s);
       }
       ru_publish_and_issue<1>(cnt, mb_ready, par_ready, mb_acc, acc_t, a_lo, wB, no_mma, lane);
       // ------------------------------------------------------------ phase C: pooled = relu(fc + b)
@@ -356,8 +402,10 @@ __global__ void __launch_bounds__(RU_THREADS, 1) render_multi_umma_kernel(bmv_re
         float pc[8];
         tmem_ld8(tcol + RU_T_FC + 8 * half, pc);
         const float4 b0 = *reinterpret_cast<const float4*>(sV + UV_BFC + 8 * half), b1 = *reinterpret_cast<const float4*>(sV + UV_BFC + 8 * half + 4);
-        ru_put(tile, RU_POOLED + half, row, fmaxf(pc[0] + b0.x, 0.f), fmaxf(pc[1] + b0.y, 0.f), fmaxf(pc[2] + b0.z, 0.f), fmaxf(pc[3] + b0.w, 0.f),
-               fmaxf(pc[4] + b1.x, 0.f), fmaxf(pc[5] + b1.y, 0.f), fmaxf(pc[6] + b1.z, 0.f), fmaxf(pc[7] + b1.w, 0.f));
+        const RuWords pw = ru_split(fmaxf(pc[0] + b0.x, 0.f), fmaxf(pc[1] + b0.y, 0.f), fmaxf(pc[2] + b0.z, 0.f), fmaxf(pc[3] + b0.w, 0.f),
+                                    fmaxf(pc[4] + b1.x, 0.f), fmaxf(pc[5] + b1.y, 0.f), fmaxf(pc[6] + b1.z, 0.f), fmaxf(pc[7] + b1.w, 0.f));
+        ru_put_tm(tcol + RU_T_POOLED + 4 * half, pw);      // A of lr0
+        ru_put(tile, RU_POOLED + half, row, pw);           // A of color.0 (shared-memory operand)
       }
       ru_publish_and_issue<2>(cnt, mb_ready, par_ready, mb_acc, acc_t, a_lo, wB, no_mma, lane);
       // ------------------------------------------------------------ phase D: hid = relu(lr0), partial sigma
@@ -377,8 +425,8 @@ __global__ void __launch_bounds__(RU_THREADS, 1) render_multi_umma_kernel(bmv_re
             h[j] = fmaxf(h[j], 0.f); h[j + 1] = fmaxf(h[j + 1], 0.f); h[j + 2] = fmaxf(h[j + 2], 0.f); h[j + 3] = fmaxf(h[j + 3], 0.f);
             a0 = fmaf(w.x, h[j], a0); a1 = fmaf(w.y, h[j + 1], a1); a2 = fmaf(w.z, h[j + 2], a2); a3 = fmaf(w.w, h[j + 3], a3);
           }
-          ru_put(tile, RU_HID + 4 * half + 2 * cb, row, h);
-          ru_put(tile, RU_HID + 4 * half + 2 * cb + 1, row, h + 8);
+          ru_put(tile, RU_HID + 4 * half + 2 * cb, row, ru_split(h));
+          ru_put(tile, RU_HID + 4 * half + 2 * cb + 1, row, ru_split(h + 8));
         }
         sig_part = (a0 + a1) + (a2 + a3);
       }
@@ -408,11 +456,15 @@ __global__ void __launch_bounds__(RU_THREADS, 1) render_multi_umma_kernel(bmv_re
           }
         }
       }
+      // the pair barrier also orders half 1's colour-accumulator loads before half 0's tcgen05.st of the next unit's
+      // operand slabs into the same lanes and columns
       tc_fence_before();
       if (half == 0) s_xe[tile_id][row] = make_float4(cl[0], cl[1], cl[2], sig_part);
       bar_sync_named(pair_bar, 64);
+      tc_fence_after();
       if (half == 1 && live) {
         const float4 o0 = s_xe[tile_id][row];
+        const float bs = sV[UV_SC + 1], b2 = sV[UV_SC + 2];
         const float c0 = fmaxf((o0.x + cl[0]) + b2, 0.f), c1 = fmaxf((o0.y + cl[1]) + b2, 0.f), c2 = fmaxf((o0.z + cl[2]) + b2, 0.f);
         const float mx = fmaxf(c0, fmaxf(c1, c2));
         const float e0 = expf(c0 - mx), e1 = expf(c1 - mx), e2 = expf(c2 - mx);

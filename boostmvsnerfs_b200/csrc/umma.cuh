@@ -31,6 +31,14 @@ __device__ __forceinline__ void umma_f16_lohi(uint32_t d_tmem, uint32_t a_lo, ui
                " tcgen05.mma.cta_group::1.kind::f16 [%0], da, db, %5, p;\n}\n"
                ::"r"(d_tmem), "r"(a_lo), "r"(a_hi), "r"(b_lo), "r"(b_hi), "r"(idesc), "n"(ACC ? 1 : 0) : "memory");
 }
+// the TS form: A from tensor memory (K-major; kind::f16: one 32-bit column holds two consecutive K values of a row, low
+// half first, so one K = 16 slab of A is 8 columns starting at a_tmem), B from shared memory as above
+template <bool ACC>
+__device__ __forceinline__ void umma_f16_ts(uint32_t d_tmem, uint32_t a_tmem, uint32_t b_lo, uint32_t b_hi, uint32_t idesc) {
+  asm volatile("{\n .reg .pred p;\n .reg .b64 db;\n setp.ne.b32 p, %5, 0;\n mov.b64 db, {%2, %3};\n"
+               " tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], db, %4, p;\n}\n"
+               ::"r"(d_tmem), "r"(a_tmem), "r"(b_lo), "r"(b_hi), "r"(idesc), "n"(ACC ? 1 : 0) : "memory");
+}
 // one K = 16 step of a split product: D (+)= A_lo B_hi + A_hi B_lo + A_hi B_hi
 __device__ __forceinline__ void umma_kstep(uint32_t d_tmem, uint32_t a_hi, uint32_t a_lbo, uint32_t a_lo_off, uint32_t b_hi,
                                            uint32_t b_lbo, uint32_t b_lo_off, uint32_t idesc, uint32_t acc) {
@@ -120,6 +128,19 @@ __device__ __forceinline__ void tmem_ld16(uint32_t taddr, float (&v)[16]) {
 #pragma unroll
   for (int i = 0; i < 16; ++i) v[i] = __uint_as_float(r[i]);
 }
+// 4 / 16 consecutive 32-bit columns of this thread's TMEM lane.  Unlike the loads these do not wait: a writer issues
+// all its stores and then tmem_wait_st() once, before it tells another thread (or the tensor core) about them.
+__device__ __forceinline__ void tmem_st4(uint32_t taddr, const uint32_t (&r)[4]) {
+  asm volatile("tcgen05.st.sync.aligned.32x32b.x4.b32 [%0], {%1,%2,%3,%4};"
+               ::"r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]) : "memory");
+}
+__device__ __forceinline__ void tmem_st16(uint32_t taddr, const uint32_t (&r)[16]) {
+  asm volatile("tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16};"
+               ::"r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]),
+                 "r"(r[8]), "r"(r[9]), "r"(r[10]), "r"(r[11]), "r"(r[12]), "r"(r[13]), "r"(r[14]), "r"(r[15]) : "memory");
+}
+__device__ __forceinline__ void tmem_wait_st() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
+
 // one warp allocates `cols` (power of two >= 32) TMEM columns; the base address lands in shared memory
 __device__ __forceinline__ void tmem_alloc(uint32_t smem_dst, uint32_t cols) {
   asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_dst), "r"(cols) : "memory");
