@@ -183,13 +183,6 @@ class Conv2dParams(C.Structure):
                 ("wfrag1x1", C.c_void_p), ("bias1x1", C.c_void_p)]
 
 
-class Conv3dSmallParams(C.Structure):
-    _fields_ = [("x", C.c_void_p), ("x_n_stride", i64), ("x_d_stride", i64), ("x_y_stride", i64), ("x_x_stride", i64),
-                ("N", i32), ("D", i32), ("H", i32), ("W", i32), ("Cin", i32), ("Cout", i32),
-                ("stride", i32), ("transposed", i32), ("relu", i32), ("out_half", i32),
-                ("wfrag", C.c_void_p), ("bias", C.c_void_p), ("skip", C.c_void_p), ("out", C.c_void_p)]
-
-
 class FpnStemParams(C.Structure):
     _fields_ = [("x", C.c_void_p), ("x_n_stride", i64), ("x_c_stride", i64), ("x_y_stride", i64), ("x_x_stride", i64),
                 ("w0", C.c_void_p), ("b0", C.c_void_p), ("wfrag1", C.c_void_p), ("b1", C.c_void_p),
@@ -227,7 +220,6 @@ ENTRY_POINTS = {
     "bmv_nerf_mlp": NerfMlpParams,
     "bmv_render_rays": RenderRaysParams,
     "bmv_render_rays_mma": RenderRaysParams,
-    "bmv_render_rays_umma": RenderRaysParams,
     "bmv_render_rays_multi": RenderMultiParams,
     "bmv_render_rays_multi_umma": RenderMultiParams,
     "bmv_cost_volume_var_img": CostVolumeImgParams,
@@ -240,7 +232,6 @@ ENTRY_POINTS = {
     "bmv_fpn_topdown_smooth": FpnFusedParams,
     "bmv_fpn_stem": FpnStemParams,
     "bmv_conv2d_k3": Conv2dParams,
-    "bmv_conv3d_small": Conv3dSmallParams,
     "bmv_frame_psnr_accumulate": FramePsnrParams,
     "bmv_frame_to_u8": FrameToU8Params,
     "bmv_frame_ssim": FrameSsimParams,
@@ -249,7 +240,7 @@ PLAIN_SYMBOLS = ("bmv_version", "bmv_last_error_string", "bmv_launch_count", "bm
                  "bmv_nerf_mlp_weight_count", "bmv_render_rays_supported", "bmv_render_rays_mma_weight_words",
                  "bmv_render_rays_umma_weight_words", "bmv_umma_selftest",
                  "bmv_conv3d_k3_weight_words", "bmv_conv3d_k3_umma_weight_words", "bmv_conv3d_k3_last_used_tma", "bmv_convT3d_k3s2_weight_words",
-                 "bmv_fpn_topdown_smooth_weight_words", "bmv_mvs_render_umma_weight_bytes", "bmv_conv2d_k3_weight_words", "bmv_conv3d_small_weight_words")
+                 "bmv_fpn_topdown_smooth_weight_words", "bmv_mvs_render_umma_weight_bytes", "bmv_conv2d_k3_weight_words")
 
 _lib = None
 
@@ -288,8 +279,6 @@ def load():
     lib.bmv_fpn_topdown_smooth_weight_words.restype = C.c_int
     lib.bmv_conv2d_k3_weight_words.restype = C.c_int
     lib.bmv_conv2d_k3_weight_words.argtypes = [C.c_int, C.c_int]
-    lib.bmv_conv3d_small_weight_words.restype = C.c_int
-    lib.bmv_conv3d_small_weight_words.argtypes = [C.c_int, C.c_int, C.c_int]
     lib.bmv_fpn_topdown_smooth_weight_words.argtypes = [C.c_int]
     lib.bmv_mvs_render_umma_weight_bytes.restype = C.c_int
     lib.bmv_sizeof_params.restype = C.c_int

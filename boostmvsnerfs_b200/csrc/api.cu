@@ -36,7 +36,6 @@ extern "C" BMV_API int bmv_sizeof_params(const char* entry) {
   if (!strcmp(entry, "bmv_nerf_mlp")) return (int)sizeof(bmv_nerf_mlp_params);
   if (!strcmp(entry, "bmv_render_rays")) return (int)sizeof(bmv_render_rays_params);
   if (!strcmp(entry, "bmv_render_rays_mma")) return (int)sizeof(bmv_render_rays_params);
-  if (!strcmp(entry, "bmv_render_rays_umma")) return (int)sizeof(bmv_render_rays_params);
   if (!strcmp(entry, "bmv_cost_volume_var_img")) return (int)sizeof(bmv_cost_volume_img_params);
   if (!strcmp(entry, "bmv_mvs_march_fetch")) return (int)sizeof(bmv_mvs_march_params);
   if (!strcmp(entry, "bmv_fpn_topdown")) return (int)sizeof(bmv_fpn_topdown_params);
@@ -46,7 +45,6 @@ extern "C" BMV_API int bmv_sizeof_params(const char* entry) {
   if (!strcmp(entry, "bmv_fpn_topdown_smooth")) return (int)sizeof(bmv_fpn_fused_params);
   if (!strcmp(entry, "bmv_fpn_stem")) return (int)sizeof(bmv_fpn_stem_params);
   if (!strcmp(entry, "bmv_conv2d_k3")) return (int)sizeof(bmv_conv2d_params);
-  if (!strcmp(entry, "bmv_conv3d_small")) return (int)sizeof(bmv_conv3d_small_params);
   if (!strcmp(entry, "bmv_mvs_render_umma")) return (int)sizeof(bmv_mvs_render_params);
   if (!strcmp(entry, "bmv_render_rays_multi")) return (int)sizeof(bmv_render_multi_params);
   if (!strcmp(entry, "bmv_render_rays_multi_umma")) return (int)sizeof(bmv_render_multi_params);

@@ -1,4 +1,4 @@
-// Packed weights of the ENeRF per-sample MLP for the tcgen05 render kernels (render_umma.cu, render_multi_umma.cu):
+// Packed weights of the ENeRF per-sample MLP for the tcgen05 render kernel (render_multi_umma.cu):
 // mlp_pack.pack_nerf_weights_umma writes this layout (CPU restatement of packing + dataflow: tests/test_umma_pack.py).
 #pragma once
 

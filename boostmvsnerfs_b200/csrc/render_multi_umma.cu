@@ -1,10 +1,11 @@
 // K3+K5 for ALL K cost-volume chains of a frame in ONE persistent launch with the per-sample MLP on the 5th-generation
 // tensor cores (tcgen05.mma, accumulators in tensor memory): the lean gather of render_multi.cu (lean_gather.cuh) in
-// front of the UMMA formulation of render_umma.cu, restructured around what bounded those two kernels.
+// front of the UMMA formulation of the first, per-chain tcgen05 render, restructured around what bounded those two kernels.
 //
 // What was measured (profiles/round2c_ncu_render_multi.csv, BMV_RM_DEBUG dissection of render_multi.cu at C2: 1.51 ms
 // = 0.42 ms gather + 1.06 ms mma.sync MLP, the two do NOT overlap: both are issue-slot work of the same 16 warps; and
-// the first tcgen05 version, render_umma.cu: 510 us per chain with ~100 MMAs per 128-sample tile each costing ~290 clk
+// the first tcgen05 version (per chain, slower than the mma.sync kernel and removed; profiles/round1l_tcgen05.md):
+// 510 us per chain with ~100 MMAs per 128-sample tile each costing ~290 clk
 // of descriptor construction inside the elected branch, i.e. the single issuing thread bounded it):
 //   * the MMAs of a phase are issued by the LAST warp of the tile to publish its operand rows (all arrive on an mbarrier,
 //     a shared-memory counter elects the last): warp-uniform code, one elected lane; every descriptor is a (low word, constant high word) pair
@@ -487,6 +488,8 @@ __global__ void __launch_bounds__(RU_THREADS, 1) render_multi_umma_kernel(bmv_re
 
 
 }  // namespace bmv
+
+extern "C" BMV_API int bmv_render_rays_umma_weight_words(void) { return bmv::UMMA_PACK_WORDS; }
 
 extern "C" BMV_API int bmv_render_rays_multi_umma(const bmv_render_multi_params* mp, bmv_stream_t stream) {
   BMV_NVTX_RANGE("bmv_render_rays_multi_umma");

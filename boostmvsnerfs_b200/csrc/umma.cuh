@@ -1,6 +1,6 @@
 // tcgen05 (UMMA) / TMEM / mbarrier PTX wrappers shared by the 5th-generation tensor-core kernels of libbmv
-// (render_umma.cu, conv3d_umma.cu).  Field layouts: cute/arch/mma_sm100_desc.hpp (CUTLASS, vendored with the toolkit
-// image) — restated here, nothing is included from it.
+// (render_multi_umma.cu, mvs_render_umma.cu, conv3d_umma.cu).  Field layouts: cute/arch/mma_sm100_desc.hpp (CUTLASS,
+// vendored with the toolkit image) — restated here, nothing is included from it.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>

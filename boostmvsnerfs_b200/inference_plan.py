@@ -115,15 +115,6 @@ class MergedHeadsCostReg(nn.Module):
     # accumulation) when the 3-level net is used: their input (conv2) and consumer (conv9T) are libbmv kernels that take
     # fp16 anyway.  Measured on B200: 144 -> 96 us for cost_reg_1, no gain for the 2-level cost_reg_0 (32 -> 31 us).
     lowres_half = True
-    # conv3 .. conv7 on libbmv's direct tensor-core kernel (csrc/conv3d_small.cu) instead of cuDNN: 5 launches instead of 7
-    # in the 3-level net, 2 in the 2-level one.  OFF: measured SLOWER on B200 (C2 frame 3.19 -> 3.28 ms; per layer 23-33 us
-    # against 12-23 us, tools/costreg_small_times.py) — without a staged tile every A fragment costs four 4-byte loads of
-    # 4 L1 wavefronts each, ~6 wavefronts per MMA; only the transposed layer + its skip add wins (23 vs 43 us).  Kept as
-    # a function-level kernel with its parity tests.
-    small_convs = False
-    # only the transposed conv7 + its skip add on that kernel (one launch instead of cuDNN's dgrad kernel + an add; the
-    # layer where the direct kernel won in the per-layer timing); needs the fp16 low-resolution route (lowres_half)
-    small_transposed = False
 
     def __init__(self, net):
         super().__init__()
@@ -170,28 +161,6 @@ class MergedHeadsCostReg(nn.Module):
             }
         return self._packed
 
-    def _small_ok(self):
-        n = self.net
-        names = ['conv3', 'conv4'] + (['conv5', 'conv6'] if n.depth_levels == 3 else [])
-        ok = all(isinstance(getattr(n, m).bn, nn.Identity) and getattr(n, m).conv.bias is not None for m in names)
-        if n.depth_levels == 3:
-            ok = ok and isinstance(n.conv7[1], nn.Identity) and n.conv7[0].bias is not None
-        return ok and tuple(n.conv3.conv.weight.shape[:2]) == (32, 16)
-
-    def _small_weights(self, device):
-        if getattr(self, '_small', None) is None or self._small['device'] != device:
-            from .mlp_pack import pack_conv3d_small
-            n = self.net
-            bias = lambda m: m.bias.detach().float().contiguous().to(device)
-            sm = {'device': device}
-            for name in ['conv3', 'conv4'] + (['conv5', 'conv6'] if n.depth_levels == 3 else []):
-                c = getattr(n, name).conv
-                sm[name] = (pack_conv3d_small(c.weight).to(device), bias(c))
-            if n.depth_levels == 3:
-                sm['conv7'] = (pack_conv3d_small(n.conv7[0].weight, transposed=True).to(device), bias(n.conv7[0]))
-            self._small = sm
-        return self._small
-
     def input_weight_scale(self, device):
         """The power of two conv0's fp16 weights are packed with (ops.volume_scale(consumer_scale=...))."""
         return self._packed_weights(device)['conv0_ws']
@@ -211,34 +180,18 @@ class MergedHeadsCostReg(nn.Module):
             s0 = ops.conv3d_k3(x, *pk['conv0'], 8, relu=True, out_dtype=h,                  # ConvBnReLU3D(C, 8)
                                in_scale=in_scale if in_scale is not None else pk['conv0_scale'])
             s1 = ops.conv3d_k3(s0, *pk['conv1'], 16, relu=True, stride=2, out_dtype=h)   # ConvBnReLU3D(8, 16, stride=2)
-            small = self.small_convs and self._small_ok()
             half_low = self.lowres_half and n.depth_levels == 3
             # ConvBnReLU3D(16, 16): fp32 where cuDNN's TF32 layers read it, fp16 when they run in fp16 too
-            s1 = ops.conv3d_k3(s1, *pk['conv2'], 16, relu=True, out_dtype=h if (half_low or small) else torch.float32)
+            s1 = ops.conv3d_k3(s1, *pk['conv2'], 16, relu=True, out_dtype=h if half_low else torch.float32)
         else:
-            half_low = small = False
+            half_low = False
             s0 = n.conv0(x)
             s1 = n.conv2(n.conv1(s0))
-        if small:
-            # conv3 .. conv7 on libbmv's direct tensor-core kernel (csrc/conv3d_small.cu): fp16 activations throughout
-            sk = self._small_weights(x.device)
-            s2 = ops.conv3d_small(ops.conv3d_small(s1, *sk['conv3'], 32, stride=2), *sk['conv4'], 32)
-            y = s2
-            if n.depth_levels == 3:
-                y = ops.conv3d_small(ops.conv3d_small(s2, *sk['conv5'], 64, stride=2), *sk['conv6'], 64)
-                y = ops.conv3d_small(y, *sk['conv7'], 32, transposed=True, relu=False, skip=s2)
-        else:
-            low = self._half_lowres() if half_low else n
-            s2 = low.conv4(low.conv3(s1))
-            y = s2
-            if n.depth_levels == 3:
-                y6 = low.conv6(low.conv5(s2))
-                if (half_low and self.small_transposed and self._small_ok() and y6.dtype == torch.float16
-                        and y6.is_contiguous(memory_format=torch.channels_last_3d)
-                        and s2.is_contiguous(memory_format=torch.channels_last_3d)):
-                    y = ops.conv3d_small(y6, *self._small_weights(x.device)['conv7'], 32, transposed=True, relu=False, skip=s2)
-                else:
-                    y = s2 + low.conv7(y6)
+        low = self._half_lowres() if half_low else n
+        s2 = low.conv4(low.conv3(s1))
+        y = s2
+        if n.depth_levels == 3:
+            y = s2 + low.conv7(low.conv6(low.conv5(s2)))
         if fast and y.stride(1) == 1 and s1.stride(1) == 1:
             y = ops.convT3d_k3s2_add(y, *pk['conv9'], 16, skip=s1, out_dtype=torch.float16)
             # the full-resolution result only feeds the fp16-operand heads convolution: store it as fp16 (TMA-staged there)

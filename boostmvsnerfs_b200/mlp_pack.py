@@ -183,8 +183,9 @@ def pack_umma_matrix(w_pad):
 
 
 def pack_nerf_weights_umma(nerf):
-    """Weights of the level-1 NeRF MLP for the tcgen05 kernel (csrc/render_umma.cu): [hi block][lo block] with the
-    six matrices in kernel order (UW_GS .. UW_CV), each in the layout of umma_operand, then the fp32 vectors.
+    """Weights of the level-1 NeRF MLP for the tcgen05 kernel (csrc/render_multi_umma.cu, csrc/nerf_umma_pack.cuh):
+    [hi block][lo block] with the six matrices in kernel order (UW_GS .. UW_CV), each in the layout of umma_operand,
+    then the fp32 vectors.
     Returns an int32 tensor (UMMA_PACK_WORDS,) on the module's device."""
     (gs, gv, wfc, l0, cs, cv), vec = _tensor_core_matrices(nerf)
     # biases ride in the MMAs: the kernel puts a 1 in a padding column of the A operand (K index 15 of
@@ -335,30 +336,6 @@ def pack_conv2d_k3_c32(weight):
             for r in range(2):
                 for e in range(2):
                     out[:, j, nt, :, r, e] = w[nt * 8 + g, half * 16 + 2 * t + 8 * r + e, :, dx].T
-    return out.reshape(-1).view(torch.int32).to(weight.device)
-
-
-def pack_conv3d_small(weight, transposed=False):
-    """Conv3d weight (Cout, Cin, 3, 3, 3) — or ConvTranspose3d weight (Cin, Cout, 3, 3, 3) with transposed=True — ->
-    int32 tensor in the order bmv_conv3d_small reads: [tap = (kd*3+ky)*3+kx][k-step][n-tile][lane = 4g+t] x {b0, b1};
-    K index kk of k-step ks is input channel ks*16 + kk, column g of n-tile nt is output channel nt*8 + g.  The transposed
-    layer uses the taps as stored (tap k maps input i to output 2i - 1 + k)."""
-    w = weight.detach().float().cpu()
-    if transposed:
-        w = w.permute(1, 0, 2, 3, 4)
-    Cout, Cin = w.shape[:2]
-    if Cin % 16 or Cout % 8 or tuple(w.shape[2:]) != (3, 3, 3):
-        raise ValueError(f"conv3d_small is not instantiated for weight {tuple(weight.shape)}")
-    w = w.half().reshape(Cout, Cin, 27)
-    KS, NT = Cin // 16, Cout // 8
-    lane = torch.arange(32)
-    g, t = lane // 4, lane % 4
-    out = torch.empty((27, KS, NT, 32, 2, 2), dtype=torch.float16)
-    for ks in range(KS):
-        for nt in range(NT):
-            for r in range(2):
-                for e in range(2):
-                    out[:, ks, nt, :, r, e] = w[nt * 8 + g, ks * 16 + 2 * t + 8 * r + e, :].T
     return out.reshape(-1).view(torch.int32).to(weight.device)
 
 

@@ -85,8 +85,9 @@ class EnerfNetwork(nn.Module):
         self.multi_chain_volume = True         # level 0: all K cost volumes in one launch, unique views warped once
         self.overlap_fpn_topdown = True        # FPN top-down steps on a side stream under the level-0 chain (inference_plan.py)
         # per-sample MLP engine of the fused render: 'umma' — tcgen05.mma with accumulators in tensor memory, all chains in
-        # one launch (render_multi_umma.cu; single chains: render_umma.cu); 'mma' — warp-level mma.sync (render_multi.cu,
-        # render_mma.cu); 'fma' — fp32 FMA (render_fused.cu).  Same fp16 hi + lo split in both tensor-core engines.
+        # one launch (render_multi_umma.cu), per-chain fallback on mma.sync (render_mma.cu: faster than a per-chain tcgen05
+        # render, profiles/round1l_tcgen05.md); 'mma' — warp-level mma.sync (render_multi.cu, render_mma.cu); 'fma' — fp32
+        # FMA (render_fused.cu).  Same fp16 hi + lo split in both tensor-core engines.
         self.mlp_engine = 'umma'
         self.host_camera_algebra = True        # 4x4 inverses etc. on the host (one D2H of ~1 KB)
         self.generate_rays = False             # True: rays of full target images are generated on the device
@@ -412,18 +413,20 @@ class EnerfNetwork(nn.Module):
         z_all = torch.empty((K, R, S), device=dev)
         if self.fused_mlp and rc.viewdir_agg and ops.render_rays_supported(Cv, Cf, V):
             engine = self.mlp_engine if (Cf == 8 and V == 3) else 'fma'
-            packed = self._packed_mlp(i, engine)
             if (engine in ('mma', 'umma') and self.multi_chain_render and state.get('depth_all') is not None and rs == 1.
                     and all(len(tr) == 3 for tr in triples) and ops.render_rays_multi_supported(feat_vol, im_feat, rgb, V)):
                 # every chain in ONE persistent launch (csrc/render_multi.cu, or render_multi_umma.cu for the tcgen05
                 # engine); view ids from device memory when the
                 # caller (FrameGraph) supplies them
+                packed = self._packed_mlp(i, engine)
                 with self._stage(f'render_fused_l{i}'):
                     ops.render_rays_multi(state['depth_all'], state['std_all'], state['nf_all'], rays, H, W, rc.depth_inv[i], S,
                                           feat_vol, im_feat, rgb, cams, triples, packed, render_scale=rs, rgb_affine=affine,
                                           ray_begin=ray_begin, n_rays=R, views_dev=self._views_dev, engine=engine,
                                           out={'raw': raw_all, 'z_vals': z_all, 'vis_mask': mask_all})
                 return {'raws': list(raw_all.unbind(0)), 'masks': list(mask_all.unbind(0)), 'zs': list(z_all.unbind(0))}
+            engine = 'fma' if engine == 'fma' else 'mma'   # per chain, both tensor-core engines run the mma.sync kernel
+            packed = self._packed_mlp(i, engine)
             self._baked_views = True               # the per-chain launches carry their view ids as kernel arguments
             with self._stage(f'render_fused_l{i}'):
                 for k in range(K):

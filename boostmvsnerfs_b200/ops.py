@@ -626,14 +626,13 @@ def render_rays(depth, std, near_far, rays, H, W, depth_inv, S, volume, im_feat,
     Returns dict(raw (n,S,4), z_vals (n,S), vis_mask (n,S) [, vis_count (n,S) int32]); `out` may
     supply preallocated contiguous tensors for any of them."""
     depth, std, near_far = _cf32(depth, "depth"), _cf32(std, "std"), _cf32(near_far, "near_far")
-    if engine not in ("fma", "mma", "umma"):
+    if engine not in ("fma", "mma"):
         raise BmvError(f"render_rays: unknown engine {engine!r}")
     w = packed_weights
-    if engine in ("mma", "umma"):
-        words = getattr(_lib.load(), f"bmv_render_rays_{engine}_weight_words")()
+    if engine == "mma":
         if not (torch.is_tensor(w) and w.is_cuda and w.dtype == torch.int32 and w.is_contiguous()
-                and w.numel() == words):
-            raise BmvError(f"render_rays(engine='{engine}'): weights must come from mlp_pack.pack_nerf_weights_{engine}")
+                and w.numel() == _lib.load().bmv_render_rays_mma_weight_words()):
+            raise BmvError("render_rays(engine='mma'): weights must come from mlp_pack.pack_nerf_weights_mma")
     else:
         w = _cf32(w, "packed_weights")
     dev = depth.device
@@ -661,7 +660,7 @@ def render_rays(depth, std, near_far, rays, H, W, depth_inv, S, volume, im_feat,
     else:
         raw = res["raw"] = torch.empty((n, S, 4), device=dev)
     rp.mlp_weights, rp.raw = w.data_ptr(), raw.data_ptr()
-    _lib.call({"mma": "bmv_render_rays_mma", "umma": "bmv_render_rays_umma"}.get(engine, "bmv_render_rays"), rp, _stream())
+    _lib.call("bmv_render_rays_mma" if engine == "mma" else "bmv_render_rays", rp, _stream())
     return res
 
 
@@ -867,40 +866,6 @@ def convT3d_k3s2_add(x, wfrag, bias, cout, skip=None, out_dtype=torch.float32):
     p.out = out.data_ptr()
     p.o_n_stride, p.o_d_stride, p.o_y_stride, p.o_x_stride = out.stride(0), out.stride(2), out.stride(3), out.stride(4)
     _lib.call("bmv_convT3d_k3s2", p, _stream())
-    return out
-
-
-def conv3d_small(x, wfrag, bias, cout, stride=1, relu=True, transposed=False, skip=None, out_dtype=torch.float16):
-    """3x3x3 convolution (+bias, +ReLU) — or ConvTranspose3d(k3, s2, p1, op1) + bias + skip with transposed=True — for
-    the low-resolution core of the cost regularisers (bmv_conv3d_small; fp16 operands, fp32 accumulation).  x fp16
-    channels_last_3d (N,Cin,D,H,W); wfrag from mlp_pack.pack_conv3d_small; skip fp16, dense, of the output's shape."""
-    if not (torch.is_tensor(x) and x.is_cuda and x.dtype == torch.float16 and x.dim() == 5 and x.stride(1) == 1):
-        raise BmvError("conv3d_small: x must be a channels_last_3d fp16 CUDA tensor (N,C,D,H,W)")
-    _on_current_device(x, "x")
-    N, Cin, D, H, W = x.shape
-    need = _lib.load().bmv_conv3d_small_weight_words(Cin, cout, int(transposed))
-    if need < 0 or wfrag.dtype != torch.int32 or wfrag.numel() != need:
-        raise BmvError(f"conv3d_small: ({Cin} -> {cout}, transposed={transposed}) not instantiated or wfrag does not match")
-    if transposed:
-        stride = 2
-        osz = (2 * D, 2 * H, 2 * W)
-    else:
-        osz = ((D - 1) // stride + 1, (H - 1) // stride + 1, (W - 1) // stride + 1)
-    out = torch.empty((N, cout) + osz, device=x.device, dtype=out_dtype, memory_format=torch.channels_last_3d)
-    p = _lib.Conv3dSmallParams()
-    p.x = x.data_ptr()
-    p.x_n_stride, p.x_d_stride, p.x_y_stride, p.x_x_stride = x.stride(0), x.stride(2), x.stride(3), x.stride(4)
-    p.N, p.D, p.H, p.W, p.Cin, p.Cout = N, D, H, W, Cin, cout
-    p.stride, p.transposed, p.relu, p.out_half = stride, int(transposed), int(relu), int(out_dtype == torch.float16)
-    p.wfrag = wfrag.data_ptr()
-    p.bias = _cf32(bias, "bias").data_ptr() if bias is not None else 0
-    if skip is not None:
-        if not (skip.is_cuda and skip.dtype == torch.float16 and tuple(skip.shape) == tuple(out.shape)
-                and skip.is_contiguous(memory_format=torch.channels_last_3d)):
-            raise BmvError(f"conv3d_small: skip must be a dense channels_last_3d fp16 tensor of shape {tuple(out.shape)}")
-        p.skip = skip.data_ptr()
-    p.out = out.data_ptr()
-    _lib.call("bmv_conv3d_small", p, _stream())
     return out
 
 

@@ -309,15 +309,9 @@ BMV_API int bmv_render_rays_supported(int Cv, int Cf, int V);
  * Instantiated for Cv=8, Cf=8, V=3 (the ENeRF level-1 MLP). */
 BMV_API int bmv_render_rays_mma(const bmv_render_rays_params* p, bmv_stream_t stream);
 BMV_API int bmv_render_rays_mma_weight_words(void);
-/* 5th-generation tensor-core variant (csrc/render_umma.cu): same contract and the same split-fp16 arithmetic,
- * every Linear layer issued as tcgen05.mma on 128-sample tiles (operands in shared memory in the UMMA
- * K-major layout, accumulators in tensor memory, read back with tcgen05.ld); two tiles ping-pong per CTA.
- * mlp_weights must come from the UMMA packing (bmv_render_rays_umma_weight_words 32-bit words). */
-BMV_API int bmv_render_rays_umma(const bmv_render_rays_params* p, bmv_stream_t stream);
-BMV_API int bmv_render_rays_umma_weight_words(void);
-/* Unit test hook for the tcgen05 plumbing (descriptors, TMEM allocation, commit, tcgen05.ld):
- * D (128,N) fp32 = A (128,K) fp32 . B^T, B (N,K) given as [hi block][lo block] of (K/8,N,8) fp16
- * (mlp_pack.pack_umma_matrix); N % 16 == 0, 16 <= N <= 256, K % 16 == 0, K <= 96.  Device pointers. */
+/* Unit test hook for the tcgen05 plumbing of csrc/umma.cuh (descriptors, TMEM allocation, commit, tcgen05.ld;
+ * csrc/umma_selftest.cu): D (128,N) fp32 = A (128,K) fp32 . B^T, B (N,K) given as [hi block][lo block] of (K/8,N,8)
+ * fp16 (mlp_pack.pack_umma_matrix); N % 16 == 0, 16 <= N <= 256, K % 16 == 0, K <= 96.  Device pointers. */
 BMV_API int bmv_umma_selftest(const float* A, const void* B_packed, float* D, int N, int K, bmv_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------
@@ -467,30 +461,6 @@ BMV_API int bmv_convT3d_k3s2(const bmv_convT3d_params* p, bmv_stream_t stream);
 BMV_API int bmv_convT3d_k3s2_weight_words(int Cin, int Cout);
 
 /* ------------------------------------------------------------------------------------------
- * 3x3x3 convolutions of the LOW-RESOLUTION core of the 3-D cost regularisers on tensor cores (fp16 operands, fp32
- * accumulation: TF32-class, same gating as bmv_conv3d_k3): conv3 / conv4 / conv5 / conv6 (padding 1, stride 1 or 2,
- * + bias, + ReLU) and the transposed conv7 (kernel 3, stride 2, padding 1, output_padding 1, + bias, + skip)
- * (reference lib/networks/enerf/cost_reg_net.py:14-24,58-75; BN folded by the caller).  Volumes of a few 10 k voxels: a
- * direct implicit GEMM without a staged tile (csrc/conv3d_small.cu).
- *   x     fp16 channels-last-3d (N,D,H,W,Cin) via strides (elements)
- *   out   DENSE channels-last-3d (N,Do,Ho,Wo,Cout), fp16 (out_half) or fp32; Do = (D-1)/stride + 1, transposed: 2D
- *   skip  optional DENSE fp16 tensor of out's shape, added after the bias (before the ReLU), or NULL
- *   wfrag bmv_conv3d_small_weight_words(Cin, Cout, transposed) words, order [tap = (kd*3+ky)*3+kx][k-step][n-tile][lane][2]
- *         (mlp_pack.pack_conv3d_small); for the transposed layer tap k maps input i to output 2i - 1 + k.
- * Instantiated: 16 -> 32, 32 -> 32, 32 -> 64, 64 -> 64; transposed 64 -> 32.
- */
-typedef struct bmv_conv3d_small_params {
-  const void* x; int64_t x_n_stride, x_d_stride, x_y_stride, x_x_stride;
-  int32_t N, D, H, W, Cin, Cout;
-  int32_t stride, transposed, relu, out_half;
-  const uint32_t* wfrag; const float* bias;
-  const void* skip;
-  void* out;
-} bmv_conv3d_small_params;
-BMV_API int bmv_conv3d_small(const bmv_conv3d_small_params* p, bmv_stream_t stream);
-BMV_API int bmv_conv3d_small_weight_words(int Cin, int Cout, int transposed);
-
-/* ------------------------------------------------------------------------------------------
  * Fused top-down step + 3x3 smoothing convolution of the feature pyramid:
  *     mid = up2x(prev) + conv1x1(lateral_in) + lat_bias   (32 channels; as bmv_fpn_topdown, exact fp32)
  *     out = conv3x3(mid, padding 1) + bias                 (Cout = 8 or 16)
@@ -598,6 +568,7 @@ BMV_API int bmv_render_rays_multi(const bmv_render_multi_params* p, bmv_stream_t
  * tensor memory, a dedicated issuer warp, two threads per sample row); mlp_weights: mlp_pack.pack_nerf_weights_umma
  * (bmv_render_rays_umma_weight_words words).  z / visibility bit-identical to bmv_render_rays_multi, raw to ~1e-5. */
 BMV_API int bmv_render_rays_multi_umma(const bmv_render_multi_params* p, bmv_stream_t stream);
+BMV_API int bmv_render_rays_umma_weight_words(void);
 
 /* ------------------------------------------------------------------------------------------
  * f4  output sinks: what the reference's evaluator / visualiser consume, produced on the device.

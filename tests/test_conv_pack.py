@@ -280,50 +280,3 @@ def test_pack_conv1x1_after_matches_the_fragment_chaining():
     ref = w1[:, :, 0, 0] @ c
     assert torch.allclose(out, ref, atol=2e-4), (out - ref).abs().max()
 
-
-@pytest.mark.parametrize("cin,cout,stride", [(16, 32, 2), (32, 32, 1), (32, 64, 2)])
-def test_pack_conv3d_small_reproduces_conv3d(cin, cout, stride):
-    """Restates csrc/conv3d_small.cu: tap (kd,ky,kx) reads input voxel o*stride - 1 + k, k-step ks channels ks*16 .. +15."""
-    g = torch.Generator().manual_seed(cin + cout)
-    w = (torch.randn((cout, cin, 3, 3, 3), generator=g) * 0.1).half().float()
-    x = torch.randn((cin, 3, 4, 7), generator=g).half().float()
-    KS, NT = cin // 16, cout // 8
-    B = unpack_b(mlp_pack.pack_conv3d_small(w), (27, KS, NT))            # [tap][ks][nt][k][n]
-    D, H, W = x.shape[1:]
-    Do, Ho, Wo = (D - 1) // stride + 1, (H - 1) // stride + 1, (W - 1) // stride + 1
-    xp = F.pad(x, (1, 1, 1, 1, 1, 1))
-    out = torch.zeros(cout, Do, Ho, Wo)
-    for kd in range(3):
-        for ky in range(3):
-            for kx in range(3):
-                tap = (kd * 3 + ky) * 3 + kx
-                a = xp[:, kd:kd + stride * Do:stride, ky:ky + stride * Ho:stride, kx:kx + stride * Wo:stride]   # [c][od][oy][ox]
-                for ks in range(KS):
-                    for nt in range(NT):
-                        out[nt * 8:(nt + 1) * 8] += torch.einsum("kn,kdyx->ndyx", B[tap, ks, nt], a[ks * 16:(ks + 1) * 16])
-    ref = F.conv3d(x[None], w, stride=stride, padding=1)[0]
-    assert torch.allclose(out, ref, atol=3e-4), (out - ref).abs().max()
-
-
-def test_pack_conv3d_small_transposed_tap_rule():
-    """Transposed layer: out[o] = sum over taps k with (o + 1 - k) even of x[(o + 1 - k) / 2] . w[k]  (per dimension)."""
-    g = torch.Generator().manual_seed(2)
-    wt = (torch.randn((16, 8, 3, 3, 3), generator=g) * 0.1).half().float()       # ConvTranspose3d layout (Cin, Cout, k, k, k)
-    x = torch.randn((16, 2, 3, 4), generator=g).half().float()
-    B = unpack_b(mlp_pack.pack_conv3d_small(wt, transposed=True), (27, 1, 1))
-    D, H, W = x.shape[1:]
-    out = torch.zeros(8, 2 * D, 2 * H, 2 * W)
-    for od in range(2 * D):
-        for oy in range(2 * H):
-            for ox in range(2 * W):
-                for kd in range(3):
-                    for ky in range(3):
-                        for kx in range(3):
-                            if (od + 1 - kd) % 2 or (oy + 1 - ky) % 2 or (ox + 1 - kx) % 2:
-                                continue
-                            i, j, k = (od + 1 - kd) // 2, (oy + 1 - ky) // 2, (ox + 1 - kx) // 2
-                            if not (0 <= i < D and 0 <= j < H and 0 <= k < W):
-                                continue
-                            out[:, od, oy, ox] += B[(kd * 3 + ky) * 3 + kx, 0, 0].T @ x[:, i, j, k]
-    ref = F.conv_transpose3d(x[None], wt, stride=2, padding=1, output_padding=1)[0]
-    assert torch.allclose(out, ref, atol=3e-4), (out - ref).abs().max()

@@ -537,72 +537,6 @@ def test_fpn_stem_fp16_output_is_the_rounded_fp32_output():
     assert torch.equal(o16, o32.half()) and torch.equal(rgb_a, rgb_b)
 
 
-# ------------------------------------------------------------------------------------------ low-resolution U-Net core (conv3d_small.cu)
-def _ref3(fn, *a, **kw):
-    prev = torch.backends.cudnn.allow_tf32
-    torch.backends.cudnn.allow_tf32 = False
-    try:
-        with torch.no_grad():
-            return fn(*a, **kw)
-    finally:
-        torch.backends.cudnn.allow_tf32 = prev
-
-
-@pytest.mark.parametrize("cin,cout,stride,dhw", [(16, 32, 2, (4, 17, 30)), (32, 32, 1, (2, 9, 21)), (32, 64, 2, (2, 9, 21)),
-                                                 (64, 64, 1, (1, 5, 19)), (16, 32, 2, (32, 34, 60))])
-@pytest.mark.parametrize("out_dtype", [torch.float16, torch.float32])
-def test_conv3d_small_vs_torch(cin, cout, stride, dhw, out_dtype):
-    from boostmvsnerfs_b200 import ops
-    from boostmvsnerfs_b200.mlp_pack import pack_conv3d_small
-    torch.manual_seed(cin + cout + dhw[1])
-    x = torch.randn(2, cin, *dhw, device="cuda").half().contiguous(memory_format=torch.channels_last_3d)
-    w = (torch.randn(cout, cin, 3, 3, 3, device="cuda") * 0.05).half().float()
-    b = torch.randn(cout, device="cuda")
-    ref = torch.relu(_ref3(torch.nn.functional.conv3d, x.float(), w, b, stride=stride, padding=1))
-    got = ops.conv3d_small(x, pack_conv3d_small(w), b, cout, stride=stride, relu=True, out_dtype=out_dtype)
-    assert got.shape == ref.shape and got.dtype == out_dtype and got.is_contiguous(memory_format=torch.channels_last_3d)
-    tol = 2e-5 if out_dtype == torch.float32 else 1e-3
-    assert (got.float() - ref).abs().max().item() <= tol * ref.abs().max().item()
-
-
-@pytest.mark.parametrize("dhw", [(1, 5, 19), (2, 17, 30)])
-def test_conv3d_small_transposed_with_skip_vs_torch(dhw):
-    from boostmvsnerfs_b200 import ops
-    from boostmvsnerfs_b200.mlp_pack import pack_conv3d_small
-    torch.manual_seed(dhw[2])
-    x = torch.randn(2, 64, *dhw, device="cuda").half().contiguous(memory_format=torch.channels_last_3d)
-    wt = (torch.randn(64, 32, 3, 3, 3, device="cuda") * 0.05).half().float()
-    b = torch.randn(32, device="cuda")
-    skip = torch.randn(2, 32, 2 * dhw[0], 2 * dhw[1], 2 * dhw[2], device="cuda").half().contiguous(memory_format=torch.channels_last_3d)
-    ref = skip.float() + _ref3(torch.nn.functional.conv_transpose3d, x.float(), wt, b, stride=2, padding=1, output_padding=1)
-    got = ops.conv3d_small(x, pack_conv3d_small(wt, transposed=True), b, 32, transposed=True, relu=False, skip=skip, out_dtype=torch.float32)
-    assert got.shape == ref.shape
-    assert (got - ref).abs().max().item() <= 2e-5 * ref.abs().max().item()
-
-
-@pytest.mark.parametrize("levels", [2, 3])
-def test_cost_reg_plan_small_convs_match_cudnn_route(levels):
-    """(Min)CostRegNet plan with conv3 .. conv7 on bmv_conv3d_small against the same plan with those layers on cuDNN (both
-    TF32-class) and against the strict fp32 module."""
-    from boostmvsnerfs_b200.inference_plan import PlanCache
-    from boostmvsnerfs_b200.modules import CostRegNet, MinCostRegNet
-    torch.manual_seed(levels)
-    net = (CostRegNet(16) if levels == 3 else MinCostRegNet(32)).cuda().eval()
-    D = 8 if levels == 3 else 16
-    x = (torch.rand(2, 16 if levels == 3 else 32, D, 24, 40, device="cuda") * 0.5).contiguous(memory_format=torch.channels_last_3d)
-    plan = PlanCache().get(f"cost_reg_{levels}", net, torch.channels_last_3d)
-    with torch.no_grad():
-        plan.small_convs = True
-        got = [t.clone() for t in plan(x)]
-        plan.small_convs = False
-        ref = plan(x)
-        strict = _ref3(net, x)
-    for a, b, s in zip(got, ref, strict):
-        assert a.shape == b.shape == s.shape
-        assert (a - s).abs().max().item() <= 1e-2 * s.abs().max().item()
-        assert (a - b).abs().max().item() <= 1e-2 * s.abs().max().item()
-
-
 def test_conv2d_k3_large_grid_uses_the_16_row_tiles():
     """The launcher picks 8-row tiles for small grids (every other conv2d test) and 16-row tiles from 900 tiles on: the
     half-resolution layers of the C2 frame.  Same arithmetic: check both routes against torch at that size."""

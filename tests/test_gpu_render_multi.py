@@ -127,8 +127,9 @@ def test_network_uses_the_multi_launch_and_matches_per_chain(monkeypatch):
     calls = []
     orig = _lib.call
     monkeypatch.setattr(_lib, "call", lambda name, p, s: (calls.append(name), orig(name, p, s))[1])
+    renders = lambda: [c for c in calls if c.startswith("bmv_render_rays")]
     a = net(dict(batch))
-    assert calls.count("bmv_render_rays_multi_umma") == 1 and "bmv_render_rays_umma" not in calls
+    assert renders() == ["bmv_render_rays_multi_umma"]
     net.mlp_engine = "mma"
     calls.clear()
     a2 = net(dict(batch))
@@ -142,6 +143,14 @@ def test_network_uses_the_multi_launch_and_matches_per_chain(monkeypatch):
         assert err <= 2e-5, (k, err)
     for k in a:
         err = float((a[k] - b[k]).abs().max()) / float(b[k].abs().max())
+        assert err <= 2e-5, (k, err)
+    # the tcgen05 engine renders single chains on the mma.sync per-chain kernel
+    net.mlp_engine = "umma"
+    calls.clear()
+    c = net(dict(batch))
+    assert renders() == ["bmv_render_rays_mma"] * 4
+    for k in a:
+        err = float((c[k] - a[k]).abs().max()) / float(a[k].abs().max())
         assert err <= 2e-5, (k, err)
 
 

@@ -1,14 +1,14 @@
-"""CPU tests of the tcgen05 weight packing (mlp_pack.pack_nerf_weights_umma) and of the dataflow of
-csrc/render_umma.cu: the packed words are read back through the same shared-memory descriptor arithmetic the
-kernel programs (start + (n/8)*SBO + (k/8)*LBO + (n%8)*16 + (k%8)*2 bytes, SBO = 128, LBO = N*16), and the six
-matrices + vectors, applied in the kernel's phase order, reproduce the torch NeRF module."""
+"""CPU tests of the tcgen05 weight packing (mlp_pack.pack_nerf_weights_umma, csrc/nerf_umma_pack.cuh) and of the
+dataflow of csrc/render_multi_umma.cu: the packed words are read back through the same shared-memory descriptor
+arithmetic the kernel programs (start + (n/8)*SBO + (k/8)*LBO + (n%8)*16 + (k%8)*2 bytes, SBO = 128, LBO = N*16), and
+the six matrices + vectors, applied in the kernel's phase order, reproduce the torch NeRF module."""
 import numpy as np
 import torch
 
 from boostmvsnerfs_b200 import mlp_pack
 from boostmvsnerfs_b200.modules import NeRF
 
-# kernel constants (csrc/render_umma.cu)
+# kernel constants (csrc/nerf_umma_pack.cuh, read by csrc/render_multi_umma.cu)
 MATS = [("GS", 32, 32), ("GV", 32, 16), ("FC", 16, 32), ("L0", 64, 32), ("CS", 64, 96), ("CV", 64, 16)]
 UW_BLOCK = sum(n * k * 2 for _, n, k in MATS)
 UV = dict(BG=0, WA=32, BFC=64, BL=80, WS=144, BC=208, W2=272, WV=336, BV=384, SC=396, TAG=400, COUNT=404)
